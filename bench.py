@@ -3,6 +3,7 @@
 samples/s, with the HBM roofline fraction and the reference's CPU path beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c5|c4|c3|c2] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for the definitions:
   value      whole-job train interactions/s, inputs + cached sort-segment plans resident in HBM;
@@ -14,6 +15,10 @@ One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for the definitio
   cpu_baseline  the oracle's torch-eager port (same ATen op sequence as the reference trainer) timed on
              the box's host cores on a bounded, proportionally scaled sample.
   torch_eager_gpu  the same port on the same GPU at full size (SURVEY.md 8d: the number the kernels must beat).
+
+--dump-outputs DIR writes what the last timed train step returned to its caller -- the six losses and the updated
+parameters (a fixed, seeded sample of the table rows) -- as DIR/<name>.npy, so that two builds can be compared
+output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -155,6 +160,30 @@ def make_tables(w, dev, U=None, I=None, seed=17373331):
         std = 0.01 if k not in ("W", "b") else 0.1
         out[k] = torch.randn(s, generator=g, device=dev, dtype=torch.float32) * std
     return out
+
+
+def dump_outputs(out_dir, hp, loss, users, items, seed=20221014):
+    """What one HotPath.train_step returned to its caller: ``losses.npy`` (the six losses, _lib.LOSS_KEYS order) and
+    every parameter after the step (call after hp.flush(): lazy user rows are current).  A table of more rows than
+    fit 8 MB is sampled -- half of the rows from the step's own batch ``users`` / ``items`` (rows its gradients
+    reached), half uniformly, from a fixed seed -- and the sampled row ids go to ``user_rows.npy`` / ``item_rows.npy``:
+    at most ~34 MB in all for D <= 64."""
+    rng = np.random.default_rng(seed)
+    cap = (8 << 20) // (4 * hp.dim)
+    arrays = {"losses": loss.cpu().numpy()}
+    for side, n, ids in (("user", hp.n_users, users), ("item", hp.n_items, items)):
+        rows = np.arange(n) if n <= cap else np.unique(np.concatenate(
+            [rng.choice(ids, cap // 2), rng.integers(0, n, cap - cap // 2)]))
+        arrays[side + "_rows"] = rows.astype(np.float64)
+        sel = torch.from_numpy(rows).to(hp.device)
+        for k in (("Uinv", "Uenv") if side == "user" else ("Iinv", "Ienv")):
+            arrays[k] = hp.params[k].index_select(0, sel).cpu().numpy()
+    for k in ("E", "W", "b"):
+        arrays[k] = hp.params[k].cpu().numpy()
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def cpu_baseline(w, threads, budget_s=25.0, scale=None, steps=12, warmup=1):
@@ -326,7 +355,7 @@ def run_reference(args, w):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    r = cpu_baseline(w, threads, budget_s=150.0, steps=args.steps, warmup=min(args.warmup, 1))
+    r = cpu_baseline(w, threads, budget_s=float("inf"), steps=args.steps, warmup=min(args.warmup, 1))
     scale = min(1.0, 262_144 / w["B"])
     label = w["name"] if scale >= 1.0 else f"1/{round(1 / scale)}-scale replica (U, I and B divided by " \
         f"{round(1 / scale)}: bounded CPU sample) of: " + w["name"]
@@ -413,6 +442,9 @@ def run_ours_single(args, w):
                                  "achieved": a, "frac": a / peak}
     # (2) headline: lazy dense Adam (bit-identical results, tests/test_gpu_lazy.py), flush inside the region
     ms, ph_ms, launches, clk = timed(not args.dense_adam)
+    if args.dump_outputs:
+        last = args.warmup + args.steps - 1
+        dump_outputs(args.dump_outputs, hp, losses[last], batches[last % nb][0], batches[last % nb][1])
     # whole step.  SURVEY.md 8d's convention (B(32D+56+8K) + 24P) charges dense Adam traffic for all P parameters; the
     # lazy path does not move those bytes, so for this leg the fraction is taken over the bytes the step's kernels
     # ACTUALLY have to move (unique-row counts of the batches): user pass (below), item pass (theta/m/v of the unique
@@ -516,7 +548,7 @@ def run_ours_single(args, w):
     consumed = [torch.cuda.Event(), torch.cuda.Event()]
     h_loss = torch.empty((2, 6)).pin_memory()
     read_back = [torch.cuda.Event(), torch.cuda.Event()]
-    e2e_steps = max(3, min(args.steps, 32))     # same amortisation of the final flush as the device-timed leg
+    e2e_steps = args.steps                      # same amortisation of the final flush as the device-timed leg
     e2e_losses = []
 
     def issue_load(s):
@@ -585,9 +617,10 @@ def run_ours_single(args, w):
         if itr:
             roof["item_pass"]["traffic"] = itr["bytes"]
     if not args.no_cpu_baseline:
-        line["cpu_baseline"] = cpu_baseline(w, os.cpu_count() or 1)
+        # host-side leg: --steps steps unless its 25 s budget runs out first ("sample" says how many ran)
+        line["cpu_baseline"] = cpu_baseline(w, os.cpu_count() or 1, steps=args.steps)
         try:
-            line["torch_eager_gpu"] = torch_eager_gpu(w, dev, dbatches[0])
+            line["torch_eager_gpu"] = torch_eager_gpu(w, dev, dbatches[0], steps=args.steps)
             line["torch_eager_gpu"]["speedup_of_value"] = line["value"] / line["torch_eager_gpu"]["value"]
         except Exception as ex:      # noqa: BLE001 -- a baseline leg must never break the bench line
             line["torch_eager_gpu"] = {"unavailable": f"{type(ex).__name__}: {ex}"[:200]}
@@ -617,7 +650,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the parity_vs_1gpu leg")
     ap.add_argument("--dense-adam", action="store_true", help="headline with plain dense Adam instead of lazy")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the losses and (sampled) parameters of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU path (--impl ours --gpus 1)")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

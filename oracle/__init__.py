@@ -14,8 +14,8 @@ Contents
 ``invpref_torch_cpu``  torch-eager CPU restatement that issues the same ATen op
                        sequence as the reference trainer (autograd + torch.optim.Adam);
                        it is what ``bench.py`` times as the CPU baseline ("port").
-``ref_shim``           imports the *live* reference from ``/root/reference`` (only in
-                       the build container) to pin the two restatements and to
+``ref_shim``           imports the *live* reference from ``oracle/_ref`` (a checkout of
+                       the original project, when present) to pin the two restatements and to
                        generate the golden fixtures under ``tests/golden/``.
 
 Parity pinning: the reference ships no tests and no golden vectors (SURVEY.md §4), so

@@ -1,9 +1,10 @@
-"""Import the LIVE reference (``/root/reference``) as a checker.  TEST INFRASTRUCTURE ONLY.
+"""Import the LIVE reference as a checker.  TEST INFRASTRUCTURE ONLY.
 
-Only usable in the build container: ``/root/reference`` does not exist on the GPU box,
-so nothing that runs there (``-m gpu`` tests, ``smoke()``, ``bench.py``) may call this.
-``matplotlib`` / ``seaborn`` are absent from the image and are pulled in by the
-reference's ``utils.py:4-5``; they are stubbed with empty modules (SURVEY.md §8c).
+The reference is a checkout of the original project (AIflowerQ/InvPref_KDD_2022, with its ``dataset/``) placed at
+``oracle/_ref`` (git-ignored: its sources are not part of this repository) or named by ``INVPREF_REFERENCE_ROOT``.
+Where it is absent the tests that use it skip, so nothing that must run everywhere (``-m gpu`` tests, ``smoke()``,
+``bench.py``) may call this.  ``matplotlib`` / ``seaborn``, which the reference's ``utils.py:4-5`` imports, are
+stubbed with empty modules where they are not installed (SURVEY.md §8c).
 """
 from __future__ import annotations
 
@@ -13,7 +14,8 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("INVPREF_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("INVPREF_REFERENCE_ROOT",
+                          os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def available() -> bool:

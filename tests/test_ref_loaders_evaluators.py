@@ -1,5 +1,5 @@
-"""CPU, build container only (needs the reference checkout): the callers either side of the hot path --
-data loaders (SURVEY.md §8f rank 3) and evaluators (ranks 1 and 4) -- against the LIVE reference on the
+"""CPU, needs a checkout of the original project at oracle/_ref (skips without it): the callers either side of the
+hot path -- data loaders (SURVEY.md §8f rank 3) and evaluators (ranks 1 and 4) -- against the LIVE reference on the
 datasets that ship with it.  Loaders: same table sizes, same arrays, same per-user mask / ground-truth / pool
 sets.  Evaluators: same metric dictionaries when both sides score with the same stub model (the ranking logic,
 masking, item-pool highlighting, NDCG / recall / precision and the MSE / RMSE / MAE formulas are what is compared;
@@ -14,7 +14,7 @@ from oracle import ref_shim
 
 DATA = os.path.join(ref_shim.REF_ROOT, "dataset")
 pytestmark = pytest.mark.skipif(not (ref_shim.available() and os.path.isdir(DATA)),
-                                reason="reference checkout not present (build container only)")
+                                reason="no checkout of the original project at oracle/_ref")
 
 
 @pytest.fixture(scope="module")
