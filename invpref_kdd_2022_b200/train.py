@@ -72,8 +72,9 @@ class _InvPrefTrainManager:
         self.const_env_tensor_list = [torch.full((n,), k, dtype=torch.int64, device=device)
                                       for k in range(self.envs_num)]                           # train.py:758-761
         # fused engine bound to the model's parameter storages; holds the Adam state (train.py:718)
-        # lazy_adam: user rows outside a batch are updated lazily (bit-identical to dense torch.optim.Adam, see
-        # HotPath); train_a_epoch flushes at the end of the epoch, train_a_batch after every call
+        # lazy_adam: user rows outside a batch are updated lazily (the same arithmetic as dense torch.optim.Adam; one-ulp
+        # exceptions from FMA contraction, DESIGN.md); train_a_epoch flushes at the end of the epoch, train_a_batch after
+        # every call
         self.engine = model.hot_path(lr=lr, lazy=lazy_adam)
         self.engine.lr = float(lr)
         # the reference's nn.Embedding raises IndexError on an id outside its table; validate the whole training
