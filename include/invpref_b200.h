@@ -380,6 +380,28 @@ int invpref_owner_adam_push(float* theta_inv, float* theta_env, float* m_inv, fl
 int invpref_peer_allreduce(float* buf, int32_t n, int32_t n_max, int32_t world, int32_t rank, float* const* peer_slots,
                            uint32_t* const* peer_flags, uint32_t* counter, int32_t* status, void* stream);
 
+/* ---- numpy's legacy global stream (np.random.randint, MT19937) continued on the device ----------------------------
+ * The reference draws its initial environments (train.py:711) and its tie-break rows (train.py:870-871, one randint per
+ * cluster batch; consecutive calls concatenate) from numpy's global RandomState.  These calls produce exactly those
+ * draws on the device and the generator state numpy would be left in, so that a caller can hand the state back to
+ * numpy (np.random.set_state) and stay on the reference's stream.
+ *
+ * invpref_mt_jump_bytes: bytes of the jump table (GF(2) matrices of T^(8 * 2^i), T = one twist of the 624-word key,
+ * 13 matrices of 49.8 MB) and of the scratch one invpref_mt_randint call needs.  Either pointer may be NULL. */
+int invpref_mt_jump_bytes(size_t* jump_bytes, size_t* ws_bytes);
+
+/* Builds the jump table into a caller buffer of at least jump_bytes (once per device; ~15 GF(2) matrix squarings). */
+int invpref_mt_build_jumps(void* jumps, size_t jump_bytes, void* stream);
+
+/* out[0..n) = np.random.randint(0, high, n) (int64, ready as perm_idx of invpref_cluster) drawn from the MT19937 state
+ * (key_in: the 624 key words on the device, pos_in: numpy's pos, 0..624 -- a fresh np.random.seed leaves 624), and
+ * key_out (624 words) / *pos_out (device int32) = the state after the call, as np.random.get_state() would report it.
+ * numpy's method for 1 <= high <= 2^32: one tempered word w per attempt, accept w & mask if <= high - 1 (mask =
+ * 2^bitlen(high - 1) - 1); high == 1 returns zeros and consumes nothing.  INVPREF_ERR_BAD_ARG for high < 1 or
+ * high > 2^32 (numpy's 64-bit path), n < 0 or pos_in outside [0, 624].  key_out must not overlap key_in. */
+int invpref_mt_randint(const uint32_t* key_in, int32_t pos_in, int64_t high, int64_t n, int64_t* out,
+                       uint32_t* key_out, int32_t* pos_out, const void* jumps, void* ws, size_t ws_bytes, void* stream);
+
 /* Number of kernels the library has launched in this process (bench.py's gpu_launches). */
 int64_t invpref_launch_count(void);
 

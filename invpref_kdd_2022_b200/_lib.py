@@ -29,7 +29,8 @@ EXPORTS = (
     "invpref_mask_scores", "invpref_hits_from_csr", "invpref_upass_supported", "invpref_plan_status",
     "invpref_check_ids", "invpref_dyn_fill", "invpref_graph_begin", "invpref_graph_end", "invpref_graph_launch",
     "invpref_graph_destroy", "invpref_graph_launches", "invpref_owner_adam_push", "invpref_eval_topk",
-    "invpref_cluster_sorted", "invpref_peer_allreduce",
+    "invpref_cluster_sorted", "invpref_peer_allreduce", "invpref_mt_jump_bytes", "invpref_mt_build_jumps",
+    "invpref_mt_randint",
 )
 # execution order; on the fused path "forward" is empty and chunks_users / rows_users are the fused user pass
 PHASES = ("plan", "forward", "chunks_users", "rows_users", "chunks_items", "rows_items", "sweep_items",
@@ -138,6 +139,9 @@ def load() -> C.CDLL:
                                       vp, vp, vp, vp, vp]
     lib.invpref_mask_scores.argtypes = [vp, i64, i64, vp, vp, vp, C.c_float, C.c_int32, vp]
     lib.invpref_hits_from_csr.argtypes = [vp, i64, C.c_int32, vp, vp, vp, vp, vp, vp]
+    lib.invpref_mt_jump_bytes.argtypes = [C.POINTER(sz), C.POINTER(sz)]
+    lib.invpref_mt_build_jumps.argtypes = [vp, sz, vp]
+    lib.invpref_mt_randint.argtypes = [vp, C.c_int32, i64, i64, vp, vp, vp, vp, vp, sz, vp]
     lib.invpref_profile_enable.argtypes = [C.c_int]
     lib.invpref_profile_read.argtypes = [C.c_int, C.POINTER(C.c_float)]
     for name in EXPORTS:

@@ -137,6 +137,36 @@ inline int make_geometry(const invpref_desc* d, Geometry* g) {
 extern long long g_launch_count;   // host-side counter (api.cu)
 inline void count_launch(int n = 1) { g_launch_count += n; }
 
+// Exclusive prefix of `v` over the CTA (blockDim.x a multiple of 32, <= 1024); *total = the CTA's sum.
+// `sm` = 33 ints of shared memory; may be reused right after the call.
+__device__ __forceinline__ int block_exclusive_scan(int v, int* total, int* sm) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    int inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int y = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += y;
+    }
+    if (lane == 31) sm[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        const int w = lane < nwarps ? sm[lane] : 0;
+        int winc = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, winc, o);
+            if (lane >= o) winc += y;
+        }
+        sm[lane] = winc - w;
+        if (lane == 31) sm[32] = winc;
+    }
+    __syncthreads();
+    const int res = inc - v + sm[warp];
+    *total = sm[32];
+    __syncthreads();
+    return res;
+}
+
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) once per kernel instantiation (and again only if a larger size is
 // asked for), not on every launch: each textual expansion owns its static.  One process drives one GPU.
 #define INVPREF_SET_SMEM_ONCE(KERNEL, BYTES)                                                                     \

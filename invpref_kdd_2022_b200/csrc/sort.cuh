@@ -40,36 +40,6 @@ inline size_t rs_scratch_bytes(int64_t n) {
 }
 inline size_t sc_scratch_bytes(int64_t n) { return align_up((size_t)(sc_tiles(n) + 1) * 4); }
 
-// Exclusive prefix of `v` over the CTA (blockDim.x a multiple of 32, <= 1024); *total = the CTA's sum.
-// `sm` = 33 ints of shared memory; may be reused right after the call.
-__device__ __forceinline__ int block_exclusive_scan(int v, int* total, int* sm) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-    int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int y = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += y;
-    }
-    if (lane == 31) sm[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        const int w = lane < nwarps ? sm[lane] : 0;
-        int winc = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int y = __shfl_up_sync(0xffffffffu, winc, o);
-            if (lane >= o) winc += y;
-        }
-        sm[lane] = winc - w;
-        if (lane == 31) sm[32] = winc;
-    }
-    __syncthreads();
-    const int res = inc - v + sm[warp];
-    *total = sm[32];
-    __syncthreads();
-    return res;
-}
-
 // ---------------------------------------------------------------------------------------------- radix sort
 __global__ void __launch_bounds__(RS_THREADS)
 rs_hist_kernel(const int32_t* __restrict__ keys, int64_t n, int shift, unsigned mask, int32_t* __restrict__ tile_hist,

@@ -28,6 +28,7 @@ import numpy as np
 import torch
 
 from ._lib import LOSS_KEYS
+from .npstream import device_randint
 from .parallel import DistDriver, ShardedBatch, ShardedTrainer, build_route_gen
 from .utils import _mean_merge_dict_func, merge_dict, transfer_loss_dict_to_line_str
 
@@ -43,7 +44,8 @@ class _ShardedInvPrefTrainManager:
                  use_recommend_re_weight: bool = True, reg_only_embed: bool = False, reg_env_embed: bool = True,
                  evaluator=None, group=None, local_rows: torch.Tensor = None, total_rows: int = None,
                  init: dict = None, seed: int = 17373331, exchange: str = "push", lazy_adam: bool = True,
-                 driver=None, rank: int = None, world: int = None, peer_sync: bool = True, use_graph: bool = True):
+                 driver=None, rank: int = None, world: int = None, peer_sync: bool = True, use_graph: bool = True,
+                 tie_break_rng: str = "numpy"):
         """Model arguments (``user_num .. factor_num``, ``reg_*``) are those of ``InvPrefExplicit/Implicit``
         (models.py:415-418): the sharded tables live in this object, not in an ``nn.Module``.  ``training_data``:
         int64 ``[n, 3]`` (user, item, score) -- the whole training set, or, with ``local_rows`` (their global row
@@ -52,7 +54,12 @@ class _ShardedInvPrefTrainManager:
         ``peer_sync``: with a peer-memory exchange, also run the step's small all-reduce and barriers over peer
         memory (``invpref_peer_allreduce``) instead of NCCL.  ``use_graph``: with push + peer_sync (a step is then
         nothing but library kernels) every epoch after the first is replayed as ONE CUDA-graph launch per rank.
-        ``driver`` / ``rank`` / ``world``: for simulated ranks (tests); default: torch.distributed."""
+        ``driver`` / ``rank`` / ``world``: for simulated ranks (tests); default: torch.distributed.
+        ``tie_break_rng``: "numpy" draws the initial environments and the tie-break rows from numpy's global stream on
+        the host, "numpy_device" draws the same values on the GPU (npstream.py), one global batch at a time."""
+        if tie_break_rng not in ("numpy", "numpy_device"):
+            raise ValueError("tie_break_rng must be 'numpy' or 'numpy_device'")
+        self.tie_break_rng = tie_break_rng
         if driver is None and world == 1:
             from .parallel import LocalDriver
             driver = LocalDriver()                                    # one rank: no process group needed
@@ -76,9 +83,15 @@ class _ShardedInvPrefTrainManager:
         self.users_tensor = data[:, 0].contiguous()                   # GLOBAL ids of the local share
         self.items_tensor = data[:, 1].contiguous()
         self.scores_tensor = data[:, 2].float().contiguous()
+        bounds = torch.arange(0, N + batch_size, batch_size, device=device).clamp_(max=N)
+        self._lo = torch.searchsorted(rows, bounds).tolist()          # local slice of every global batch
         # train.py:711: the global draw, identical on every rank; the local share keeps its rows
-        envs_all = np.random.randint(0, self.envs_num, N)
-        self.envs = torch.from_numpy(envs_all).to(device)[rows].contiguous()
+        if tie_break_rng == "numpy_device":
+            self.envs = torch.cat([self._global_draw(env_num, b, min(N, (b + 1) * batch_size) - b * batch_size,
+                                                     batch_size) for b in range(len(self._lo) - 1)])
+        else:
+            envs_all = np.random.randint(0, self.envs_num, N)
+            self.envs = torch.from_numpy(envs_all).to(device)[rows].contiguous()
         self.cluster_interval, self.evaluate_interval = cluster_interval, evaluate_interval
         self.batch_size, self.epochs, self.lr = batch_size, epochs, lr
         self.invariant_coe, self.env_aware_coe, self.env_coe = invariant_coe, env_aware_coe, env_coe
@@ -101,8 +114,6 @@ class _ShardedInvPrefTrainManager:
         self.cluster_use_random_sort = cluster_use_random_sort
         self.evaluator = evaluator
         # ---- the sharded engine ----
-        bounds = torch.arange(0, N + batch_size, batch_size, device=device).clamp_(max=N)
-        self._lo = torch.searchsorted(rows, bounds).tolist()          # local slice of every global batch
         per_rank = max(self._lo[b + 1] - self._lo[b] for b in range(self.batch_num))
         if driver is None and self.world > 1:
             # the symmetric-memory buffer must have the same layout (hence the same size) on every rank: size the
@@ -279,7 +290,9 @@ class _ShardedInvPrefTrainManager:
         for b, sb in enumerate(self._batches):
             lo, hi = self._lo[b], self._lo[b + 1]
             perm = None
-            if self.cluster_use_random_sort:          # the global draw of train.py:870-871, this rank's rows of it
+            if self.cluster_use_random_sort and self.tie_break_rng == "numpy_device":
+                perm = self._global_draw(self.eps_random_tensor.shape[0], b, sb.global_batch, self.batch_size)
+            elif self.cluster_use_random_sort:        # the global draw of train.py:870-871, this rank's rows of it
                 idx = np.random.randint(0, self.eps_random_tensor.shape[0], sb.global_batch)
                 g_lo = b * self.batch_size
                 perm = torch.from_numpy(idx.astype(np.int64)).to(self.device)[self.rows[lo:hi] - g_lo].contiguous()
@@ -292,6 +305,12 @@ class _ShardedInvPrefTrainManager:
         self.envs = new_envs
         self._hist = acc[:self.envs_num].clone()
         return int(acc[self.envs_num].item())
+
+    def _global_draw(self, high: int, b: int, count: int, batch_size: int) -> torch.Tensor:
+        """np.random.randint(0, high, count) for global batch b, drawn on the device; this rank's rows of it."""
+        d = device_randint(high, count, self.device)
+        lo, hi = self._lo[b], self._lo[b + 1]
+        return d[self.rows[lo:hi] - b * batch_size].contiguous()
 
     def stat_envs(self) -> dict:
         """train.py:945-957 with the GLOBAL histogram (one all-reduce of K counters)."""

@@ -51,7 +51,8 @@ def run_main(implicit, device, model_config, train_config, evaluate_config, data
         lr=tc['lr'], invariant_coe=tc['invariant_coe'], env_aware_coe=tc['env_aware_coe'], env_coe=tc['env_coe'],
         L2_coe=tc['L2_coe'], L1_coe=tc['L1_coe'], alpha=tc['alpha'], use_class_re_weight=tc['use_class_re_weight'],
         test_begin_epoch=tc['test_begin_epoch'], begin_cluster_epoch=tc['begin_cluster_epoch'],
-        stop_cluster_epoch=tc['stop_cluster_epoch'], use_recommend_re_weight=tc['use_recommend_re_weight'])
+        stop_cluster_epoch=tc['stop_cluster_epoch'], use_recommend_re_weight=tc['use_recommend_re_weight'],
+        tie_break_rng=tc.get('tie_break_rng', 'numpy'))
     train_tuple, test_tuple, cluster_tuple = train_manager.train(silent=silent, auto=auto)
     merged = merge_dict(test_tuple[0], _show_me_a_list_func)
     metric = evaluate_config['eval_metric']
@@ -97,11 +98,17 @@ def cli(module, implicit, shape=None):
                     help='synthetic interactions of the config\'s shape (train.csv of MovieLens / MIND is not '
                          'in the reference checkout)')
     ap.add_argument('--dataset-root', default=global_config.DATASET_PATH)
+    ap.add_argument('--numpy-stream-on-device', action='store_true',
+                    help='draw the initial environments and the cluster tie-break rows from numpy\'s global stream '
+                         'on the GPU: the same values and the same numpy state as the host draws, without their '
+                         'host time')
     args = ap.parse_args()
     device = default_device()
     train_config = dict(module.TRAIN_CONFIG)
     if args.epochs is not None:
         train_config['epochs'] = args.epochs
+    if args.numpy_stream_on_device:
+        train_config['tie_break_rng'] = 'numpy_device'
     path = args.dataset_root + module.DATASET_PATH
     Loader = dl.YahooImplicitBCELossDataLoader if implicit else dl.ExplicitDataLoader
     if args.synthetic or not os.path.isfile(os.path.join(path, 'train.csv')):

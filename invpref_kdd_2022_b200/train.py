@@ -7,7 +7,8 @@ Kept from the reference, because results depend on them:
   * batches are the sequential, unshuffled slices of ``utils.mini_batch`` (utils.py:12-19);
   * the initial environments come from ``np.random.randint`` at construction (train.py:711) and the
     tie-break indices from one ``np.random.randint(0, K!, b)`` per cluster batch (train.py:870-871), drawn
-    on the host from numpy's global stream in the reference's order;
+    from numpy's global stream in the reference's order -- on the host, or with ``tie_break_rng="numpy_device"``
+    the same values on the GPU (npstream.py);
   * alpha schedule (train.py:891-894), stat_envs weighting (train.py:945-957), loss-dict keys and the
     per-epoch ``np.mean`` of per-batch python floats (utils.py:181-183).
 """
@@ -20,6 +21,7 @@ import numpy as np
 import torch
 
 from ._lib import LOSS_KEYS
+from .npstream import device_randint
 from .utils import _mean_merge_dict_func, merge_dict, mini_batch, transfer_loss_dict_to_line_str
 
 
@@ -36,8 +38,9 @@ class _InvPrefTrainManager:
             use_graph: bool = True, plan_cache_bytes: int = 16 << 30, sorted_cluster: bool = False,
             tie_break_rng: str = "numpy"
     ):
-        if tie_break_rng not in ("numpy", "device"):
-            raise ValueError("tie_break_rng must be 'numpy' (the reference's host stream, train.py:870-871) or 'device'")
+        if tie_break_rng not in ("numpy", "device", "numpy_device"):
+            raise ValueError("tie_break_rng must be 'numpy' (the reference's host stream, train.py:870-871), "
+                             "'numpy_device' (the same stream drawn on the GPU) or 'device'")
         self.tie_break_rng = tie_break_rng
         self.model = model
         self.evaluator = evaluator
@@ -48,7 +51,10 @@ class _InvPrefTrainManager:
         self.users_tensor = training_data[:, 0].contiguous().to(device)
         self.items_tensor = training_data[:, 1].contiguous().to(device)
         self.scores_tensor = training_data[:, 2].float().contiguous().to(device)
-        self.envs = torch.LongTensor(np.random.randint(0, self.envs_num, n)).to(device)       # train.py:711
+        if tie_break_rng == "numpy_device":
+            self.envs = device_randint(self.envs_num, n, device)                                 # train.py:711
+        else:
+            self.envs = torch.LongTensor(np.random.randint(0, self.envs_num, n)).to(device)   # train.py:711
         self.cluster_interval, self.evaluate_interval = cluster_interval, evaluate_interval
         self.batch_size, self.epochs = batch_size, epochs
         self.lr = lr
@@ -297,7 +303,9 @@ class _InvPrefTrainManager:
     def cluster_a_batch(self, batch_users_tensor, batch_items_tensor, batch_scores_tensor) -> torch.Tensor:
         """train.py:846-879 for one batch (draws its tie-break indices like the reference)."""
         perm = None
-        if self.cluster_use_random_sort:
+        if self.cluster_use_random_sort and self.tie_break_rng == "numpy_device":
+            perm = device_randint(self.eps_random_tensor.shape[0], batch_users_tensor.shape[0], self.device)
+        elif self.cluster_use_random_sort:
             idx = np.random.randint(0, self.eps_random_tensor.shape[0], batch_users_tensor.shape[0])
             perm = torch.from_numpy(idx.astype(np.int64)).to(self.device)
         new_envs, _, _ = self.engine.cluster(batch_users_tensor.contiguous(), batch_items_tensor.contiguous(),
@@ -316,6 +324,9 @@ class _InvPrefTrainManager:
             # decide between environments whose distances agree to ~1e-10 (train.py:763-769), but numpy's sequential
             # Mersenne-Twister stream costs ~10 ns per sample on the host -- 40 of the 53 ms of a MIND-sized cluster()
             perm = torch.randint(0, self.eps_random_tensor.shape[0], (n,), device=self.device)
+        elif self.cluster_use_random_sort and self.tie_break_rng == "numpy_device":
+            # the per-batch draws concatenate into one draw of n: the same values, numpy's state advanced the same
+            perm = device_randint(self.eps_random_tensor.shape[0], n, self.device)
         elif self.cluster_use_random_sort:
             draws = [np.random.randint(0, self.eps_random_tensor.shape[0], min(self.batch_size, n - lo))
                      for lo in range(0, n, self.batch_size)]
