@@ -11,7 +11,7 @@ import os
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# INVPREF_LIB: another build of the same library (A/B runs of kernel variants in bench.py; see tools/build_variants.sh)
+# INVPREF_LIB: load another build of the same library instead of the in-tree one
 LIB_PATH = os.environ.get("INVPREF_LIB") or os.path.join(_HERE, "libinvpref_b200.so")
 
 MAX_ENVS = 8

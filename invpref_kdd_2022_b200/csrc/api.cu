@@ -1,6 +1,5 @@
 // extern "C" entry points of libinvpref_b200.so (see include/invpref_b200.h).
 #include <math.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -63,15 +62,6 @@ void carve_plan(const invpref_desc* d, int64_t B, char* plan, PlanSide* pu, Plan
     *pi = carve_plan_side(plan + plan_side_bytes(Bp, d->n_users), Bp, d->n_items);
     pu->B = B;
     pi->B = B;
-}
-
-// INVPREF_FUSED=0 selects the unfused path (forward kernel + separate user-side rows kernel) for A/B runs
-bool use_fused_user_pass(const Geometry& g) {
-    static const bool enabled = [] {
-        const char* e = getenv("INVPREF_FUSED");
-        return !(e && e[0] == '0');
-    }();
-    return enabled && upass_supported(g);
 }
 
 int build_plan_impl(const invpref_desc* d, const int64_t* users, const int64_t* items, int64_t B, char* plan,
@@ -240,7 +230,7 @@ int invpref_upass_supported(const invpref_desc* desc) {
     Geometry g;
     int rc = make_geometry(desc, &g);
     if (rc != INVPREF_OK) return rc;
-    return use_fused_user_pass(g) ? 1 : 0;
+    return upass_supported(g) ? 1 : 0;
 }
 
 int invpref_plan_status(const invpref_desc* desc, const void* plan, int64_t B, void* stream) {
@@ -335,7 +325,7 @@ int invpref_train_step(const invpref_desc* desc, const invpref_params* pin, invp
     const bool lazy = adam->user_last_step != nullptr;
     if (lazy) {
         // lazy user rows: fused pass only, in place, Adam (not export), schedule table with room for this step
-        if (exp_u || !adam->sched || hyper->step >= adam->sched_cap || !use_fused_user_pass(g) ||
+        if (exp_u || !adam->sched || hyper->step >= adam->sched_cap || !upass_supported(g) ||
             pin->Uinv != pout->Uinv || pin->Uenv != pout->Uenv || (hyper->flags & INVPREF_DEFER_USER_SWEEP))
             return INVPREF_ERR_BAD_ARG;
     }
@@ -395,7 +385,7 @@ int invpref_train_step(const invpref_desc* desc, const invpref_params* pin, invp
 
     const int P = fwd_partial_floats(g);
     int n_partials;
-    if (use_fused_user_pass(g)) {
+    if (upass_supported(g)) {
         // (1)+(2)+(3u)+(4u) fused USER PASS: forward, losses, user-side segment reduce, Adam on user rows
         UserPassArgs up;
         up.side = su;

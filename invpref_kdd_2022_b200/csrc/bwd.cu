@@ -202,10 +202,7 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_kernel(BwdSideArgs a) {
     }
 }
 
-#ifndef INVPREF_RING_DEPTH
-#define INVPREF_RING_DEPTH 4
-#endif
-constexpr int RING = INVPREF_RING_DEPTH;   // interactions in flight per group (ring kernels)
+constexpr int RING = 4;   // interactions in flight per group (ring kernels); deeper rings measured slower (DESIGN.md §3)
 
 // One interaction of the ring kernels: its g-pack (shared by the group) and the two partner-row slices this
 // lane staged, accumulated exactly as accumulate_range does.
@@ -481,7 +478,6 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_ring_kernel(BwdSideArgs a, 
     for (int q = 0; q < RING - 1; ++q) produce();
 
     // ---- consumer: the same ranges, segment by segment ----
-#if INVPREF_ITEM_STAGE_OWN
     auto request_own = [&](int64_t row_) {     // theta / m / v rows of one item row -> the six slots behind the ring
         stage_row_async<VEC, NV>(ring, RING * 2 + 0, a.own_inv_in, row_, D, lane);
         stage_row_async<VEC, NV>(ring, RING * 2 + 1, a.own_env_in, row_, D, lane);
@@ -492,7 +488,6 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_ring_kernel(BwdSideArgs a, 
             stage_row_async<VEC, NV>(ring, RING * 2 + 5, a.v_env, row_, D, lane);
         }
     };
-#endif
     int rslot = 0, rgs = 0;
     int csa_n = 0, csb_n = 0;      // bounds of the consumer's next range
     if (g < NR) { csa_n = range_start[g]; csb_n = range_start[g + 1]; }
@@ -513,20 +508,11 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_ring_kernel(BwdSideArgs a, 
                 if (c1 - c0 > HOT_CHUNKS) continue;           // reduced by a whole CTA above
             }
             Row<VEC, NV> th_i, th_e, m_i, m_e, v_i, v_e;
-#if INVPREF_ITEM_STAGE_OWN
             // own rows: global -> shared now (slots behind the ring; each lane its own slice), read after the loop.
-            // The copies join the cp.async group of the next commit (the first produce() below).
+            // The copies join the cp.async group of the next commit (the first produce() below).  Register loads
+            // issued here instead would carry their scoreboard wait on the interaction loop's first branch, where
+            // ncu found 37 % of the kernel's warp samples (DESIGN.md §3).
             request_own(row);
-#else
-            load_row<VEC, NV>(th_i, a.own_inv_in, row, D, lane);
-            load_row<VEC, NV>(th_e, a.own_env_in, row, D, lane);
-            if (EPI == EPI_ADAM) {
-                load_row<VEC, NV, true>(m_i, a.m_inv, row, D, lane);
-                load_row<VEC, NV, true>(m_e, a.m_env, row, D, lane);
-                load_row<VEC, NV, true>(v_i, a.v_inv, row, D, lane);
-                load_row<VEC, NV, true>(v_e, a.v_env, row, D, lane);
-            }
-#endif
             Row<VEC, NV> gi, ge;
 #pragma unroll
             for (int x = 0; x < NV * VEC; ++x) { gi.x[x] = 0.f; ge.x[x] = 0.f; }
@@ -538,10 +524,8 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_ring_kernel(BwdSideArgs a, 
 #pragma unroll
                     for (int x = 0; x < NV * VEC; ++x) { gi.x[x] += pi.x[x]; ge.x[x] += pe.x[x]; }
                 }
-#if INVPREF_ITEM_STAGE_OWN
                 cp_async_commit();       // no produce() on this path: the own rows get a group of their own
                 cp_async_wait<0>();
-#endif
             } else {
                 for (int k = beg; k < end; ++k) {
                     produce();
@@ -551,20 +535,17 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_ring_kernel(BwdSideArgs a, 
                     if (++rslot == RING) rslot = 0;
                     if (++rgs == RING + 1) rgs = 0;
                 }
-#if INVPREF_ITEM_STAGE_OWN
                 // The own rows travel in the group of the segment's FIRST produce(); len - 1 groups were committed after
                 // it.  A loop of RING or more interactions has waited for it already (wait<RING - 1> after its last
                 // produce); a shorter one allows exactly the younger groups to stay pending.
                 {
                     const int len = end - beg;
                     if (len == 1) cp_async_wait<0>();
-                    else if (len == 2) cp_async_wait<(RING > 1 ? 1 : 0)>();
-                    else if (len == 3) cp_async_wait<(RING > 2 ? 2 : RING - 1)>();
-                    else if (len < RING) cp_async_wait<0>();      // deeper rings (A/B builds): be conservative
+                    else if (len == 2) cp_async_wait<1>();
+                    else if (len == 3) cp_async_wait<2>();
+                    else if (len < RING) cp_async_wait<0>();      // any other loop shorter than the ring: wait for all
                 }
-#endif
             }
-#if INVPREF_ITEM_STAGE_OWN
             read_staged_row<VEC, NV>(th_i, ring, RING * 2 + 0, D, lane);
             read_staged_row<VEC, NV>(th_e, ring, RING * 2 + 1, D, lane);
             if (EPI == EPI_ADAM) {
@@ -573,7 +554,6 @@ __global__ void __launch_bounds__(BLOCK, 3) bwd_rows_ring_kernel(BwdSideArgs a, 
                 read_staged_row<VEC, NV>(v_i, ring, RING * 2 + 4, D, lane);
                 read_staged_row<VEC, NV>(v_e, ring, RING * 2 + 5, D, lane);
             }
-#endif
             finish_row<VEC, NV, EPI>(a, row, (float)(end - beg), th_i, th_e, m_i, m_e, v_i, v_e, gi, ge, lane, D);
         }
     }
@@ -812,22 +792,14 @@ inline int grid_groups(int64_t n, int max_blocks) {
 
 }  // namespace
 
-static bool ring_enabled() {
-    static const bool enabled = [] {
-        const char* e = getenv("INVPREF_RING");   // INVPREF_RING=0: register-only rows / chunks kernels (A/B runs)
-        return !(e && e[0] == '0');
-    }();
-    return enabled;
-}
-
-static size_t ring_smem(const Geometry& g) {   // E, W, g-pack slots, the ring of partner rows (+ six own-row slots)
+static size_t ring_smem(const Geometry& g) {   // E, W, g-pack slots, the ring of partner rows + six own-row slots
     return ((size_t)ring_align_up(((2 * g.K * g.D + 3) & ~3) + GROUPS_PER_BLOCK * (RING + 1) * 12) +
-            (size_t)(RING * 2 + (INVPREF_ITEM_STAGE_OWN ? 6 : 0)) * g.NV * g.VEC * BLOCK) * sizeof(float);
+            (size_t)(RING * 2 + 6) * g.NV * g.VEC * BLOCK) * sizeof(float);
 }
 
 int launch_bwd_chunks(const Geometry& g, const BwdSideArgs& a, cudaStream_t stream) {
     const bool stash = a.stash != nullptr;
-    if (ring_enabled() && g.NV * g.VEC <= 4) {
+    if (g.NV * g.VEC <= 4) {
         const size_t smem = ring_smem(g);
         // chunk c goes to CTA c % grid: one CTA per SM first, up to three
         int64_t need = a.plan.max_chunks;
@@ -859,23 +831,23 @@ int launch_bwd_chunks(const Geometry& g, const BwdSideArgs& a, cudaStream_t stre
         count_launch();
         return cudaGetLastError() == cudaSuccess ? INVPREF_OK : INVPREF_ERR_CUDA;
     }
+    // wider row slices: VEC = 4 with NV = 2 or 4
     size_t smem = (size_t)2 * g.K * g.D * sizeof(float);
     int grid = grid_groups(a.plan.max_chunks, 148 * 8);
-    if (stash) {
-#define CALL(V, N) bwd_chunks_kernel<V, N, true><<<grid, BLOCK, smem, stream>>>(a)
-        INVPREF_DISPATCH_VN(g, CALL);
+#define CALL(V, N)                                                                                               \
+    do {                                                                                                         \
+        if (stash) bwd_chunks_kernel<V, N, true><<<grid, BLOCK, smem, stream>>>(a);                              \
+        else bwd_chunks_kernel<V, N, false><<<grid, BLOCK, smem, stream>>>(a);                                   \
+    } while (0)
+    if (g.NV == 2) CALL(4, 2);
+    else CALL(4, 4);
 #undef CALL
-    } else {
-#define CALL(V, N) bwd_chunks_kernel<V, N, false><<<grid, BLOCK, smem, stream>>>(a)
-        INVPREF_DISPATCH_VN(g, CALL);
-#undef CALL
-    }
     count_launch();
     return cudaGetLastError() == cudaSuccess ? INVPREF_OK : INVPREF_ERR_CUDA;
 }
 
 static bool use_ring(const Geometry& g, int epi) {
-    return ring_enabled() && g.NV * g.VEC <= 4 && (epi == EPI_ADAM || epi == EPI_EXPORT);
+    return g.NV * g.VEC <= 4 && (epi == EPI_ADAM || epi == EPI_EXPORT);
 }
 
 int launch_bwd_rows(const Geometry& g, const BwdSideArgs& a, int epi, cudaStream_t stream) {
@@ -915,21 +887,16 @@ int launch_bwd_rows(const Geometry& g, const BwdSideArgs& a, int epi, cudaStream
     }
     size_t smem = (size_t)2 * g.K * g.D * sizeof(float);
     int grid = grid_groups(a.plan.max_seg, 148 * 8);
-    if (epi == EPI_ADAM && stash) {
-#define CALL(V, N) bwd_rows_kernel<V, N, EPI_ADAM, true><<<grid, BLOCK, smem, stream>>>(a)
-        INVPREF_DISPATCH_VN(g, CALL);
-#undef CALL
-    } else if (epi == EPI_ADAM) {
-#define CALL(V, N) bwd_rows_kernel<V, N, EPI_ADAM, false><<<grid, BLOCK, smem, stream>>>(a)
-        INVPREF_DISPATCH_VN(g, CALL);
-#undef CALL
-    } else if (epi == EPI_EXPORT && stash) {
-#define CALL(V, N) bwd_rows_kernel<V, N, EPI_EXPORT, true><<<grid, BLOCK, smem, stream>>>(a)
-        INVPREF_DISPATCH_VN(g, CALL);
-#undef CALL
-    } else if (epi == EPI_EXPORT) {
-#define CALL(V, N) bwd_rows_kernel<V, N, EPI_EXPORT, false><<<grid, BLOCK, smem, stream>>>(a)
-        INVPREF_DISPATCH_VN(g, CALL);
+    if (epi == EPI_ADAM || epi == EPI_EXPORT) {   // wider row slices (use_ring): VEC = 4 with NV = 2 or 4
+#define CALL(V, N)                                                                                               \
+    do {                                                                                                         \
+        if (epi == EPI_ADAM && stash) bwd_rows_kernel<V, N, EPI_ADAM, true><<<grid, BLOCK, smem, stream>>>(a);   \
+        else if (epi == EPI_ADAM) bwd_rows_kernel<V, N, EPI_ADAM, false><<<grid, BLOCK, smem, stream>>>(a);      \
+        else if (stash) bwd_rows_kernel<V, N, EPI_EXPORT, true><<<grid, BLOCK, smem, stream>>>(a);               \
+        else bwd_rows_kernel<V, N, EPI_EXPORT, false><<<grid, BLOCK, smem, stream>>>(a);                         \
+    } while (0)
+        if (g.NV == 2) CALL(4, 2);
+        else CALL(4, 4);
 #undef CALL
     } else {
 #define CALL(V, N) bwd_rows_kernel<V, N, EPI_ACCUM, false><<<grid, BLOCK, smem, stream>>>(a)

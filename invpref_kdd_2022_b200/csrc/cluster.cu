@@ -40,21 +40,6 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
     __shared__ unsigned long long sHist[INVPREF_MAX_ENVS + 1];   // [K] histogram, [8] diff
     const int tid = threadIdx.x, lane = tid & (GROUP - 1);
     const unsigned gmask = group_mask();
-    // BULK (A/B switch INVPREF_CLUSTER_BULK, 16-byte-per-lane rows only): a sample's four rows are copied with ONE
-    // cp.async.bulk per row (UBLKCP; issued by lane 0 of the group, the row lands in the same 16 consecutive lane
-    // slots) and complete on one mbarrier per (group, ring slot) instead of cp.async.wait_group.
-#if INVPREF_CLUSTER_BULK
-    constexpr bool BULK = (VEC == 4 && NV == 1);
-#else
-    constexpr bool BULK = false;
-#endif
-    __shared__ __align__(8) unsigned long long sBar[GROUPS_PER_BLOCK][4];
-    if (BULK && lane == 0) {
-#pragma unroll
-        for (int q = 0; q < ST; ++q)
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&sBar[tid >> 4][q])) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
     for (int t = tid; t < KD; t += BLOCK) sE[t] = a.E[t];
     for (int t = tid; t < eps_rows_smem * K; t += BLOCK) sEps[t] = a.eps_table[t];
     if (tid <= INVPREF_MAX_ENVS) sHist[tid] = 0ull;
@@ -75,29 +60,11 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
     const int64_t stride = (int64_t)gridDim.x * GROUPS_PER_BLOCK;
     const int64_t n0 = (int64_t)blockIdx.x * GROUPS_PER_BLOCK + (tid >> 4);
     auto issue = [&](int slot, int64_t u, int64_t it) {
-        if (BULK) {
-            __syncwarp(gmask);                       // every lane of the group is done reading this slot's last rows
-            if (lane == 0) {
-                const uint32_t bar = smem_addr(&sBar[tid >> 4][slot]);
-                const uint32_t bytes = (uint32_t)D * 4u;
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(4u * bytes)
-                             : "memory");
-                const float* src[4] = {a.Uinv + u * D, a.Iinv + it * D, a.Uenv + u * D, a.Ienv + it * D};
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    const uint32_t dst = smem_addr(ring + ((size_t)(slot * 4 + r) * BLOCK + (tid & ~(GROUP - 1))) * VEC);
-                    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                                 ::"r"(dst), "l"(src[r]), "r"(bytes), "r"(bar) : "memory");
-                }
-            }
-            return;
-        }
         stage_row_async<VEC, NV>(ring, slot * 4 + 0, a.Uinv, u, D, lane);
         stage_row_async<VEC, NV>(ring, slot * 4 + 1, a.Iinv, it, D, lane);
         stage_row_async<VEC, NV>(ring, slot * 4 + 2, a.Uenv, u, D, lane);
         stage_row_async<VEC, NV>(ring, slot * 4 + 3, a.Ienv, it, D, lane);
     };
-    uint32_t phase = 0;                              // BULK: parity of the current use of the ring slots
     // ids are below 2^31 (make_geometry): only the low word of each int64 is loaded.  They run TWO iterations
     // ahead of the row requests (one was not enough: the request stalled on its own ids, ncu round 1).
     const int32_t* __restrict__ users_lo = reinterpret_cast<const int32_t*>(a.users);
@@ -138,29 +105,11 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
         cp_async_commit();
         uq = uq2; iq = iq2;
         if (n + (ST + 1) * stride < a.B) { uq2 = users_lo[2 * (n + (ST + 1) * stride)]; iq2 = items_lo[2 * (n + (ST + 1) * stride)]; }
-#if INVPREF_CLUSTER_L2_PREFETCH
-        // the rows that will be requested NEXT iteration (ids already in uq / iq): into L2 now, one line per lane
-        if (n + ST * stride < a.B && lane < 8) {
-            const int t = lane >> 1, half = lane & 1;
-            const float* tab = (t == 0) ? a.Uinv : ((t == 1) ? a.Iinv : ((t == 2) ? a.Uenv : a.Ienv));
-            const int64_t rr = (t & 1) ? iq : uq;
-            if (half * 32 < D) prefetch_l2(tab + rr * D + half * 32);
-        }
-#endif
         const float y = __int_as_float(__shfl_sync(gmask, sc, gbase));
         const int pidx = __shfl_sync(gmask, sc, gbase + 1);
         const int old = __shfl_sync(gmask, sc, gbase + 2);
         if (n + stride < a.B) sc = load_scalars(n + stride);
-        if (BULK) {
-            const uint32_t bar = smem_addr(&sBar[tid >> 4][slot]);
-            uint32_t ok;
-            do {
-                asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                             : "=r"(ok) : "r"(bar), "r"(phase) : "memory");
-            } while (!ok);
-        } else {
-            cp_async_wait<ST - 1>();
-        }
+        cp_async_wait<ST - 1>();
         Row<VEC, NV> ra, rc, rue, rie;
         read_staged_row<VEC, NV>(ra, ring, slot * 4 + 0, D, lane);
         read_staged_row<VEC, NV>(rc, ring, slot * 4 + 1, D, lane);
@@ -220,7 +169,7 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
             for (int k = 0; k < KT; ++k) cnt[k] += (arg == k) ? 1u : 0u;
             if (has_d && old != arg) ++ndiff;
         }
-        if (++slot == ST) { slot = 0; phase ^= 1u; }
+        if (++slot == ST) slot = 0;
     }
     cp_async_wait<0>();
     if (lane == 0) {
@@ -329,15 +278,6 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
         cp_async_commit();
         uq = uq2; iq = iq2;
         if (n + (ST + 1) * stride < B_end) { uq2 = users_lo[n + (ST + 1) * stride]; iq2 = items_lo[n + (ST + 1) * stride]; }
-#if INVPREF_CLUSTER_L2_PREFETCH
-        // the rows that will be requested NEXT iteration (ids already in uq / iq): into L2 now, one line per lane
-        if (n + ST * stride < B_end && lane < 8) {
-            const int t = lane >> 1, half = lane & 1;
-            const float* tab = (t == 0) ? a.Uinv : ((t == 1) ? a.Iinv : ((t == 2) ? a.Uenv : a.Ienv));
-            const int64_t rr = (t & 1) ? iq : uq;
-            if (half * 32 < D) prefetch_l2(tab + rr * D + half * 32);
-        }
-#endif
         const float y = __int_as_float(__shfl_sync(gmask, sc, gbase));
         const int pidx = __shfl_sync(gmask, sc, gbase + 1);
         const int old = __shfl_sync(gmask, sc, gbase + 2);

@@ -6,45 +6,6 @@
 
 #include "invpref_b200.h"
 
-// A/B switches of the round-2 instruction diet (compile-time; -DNAME=0 builds the round-1 arithmetic)
-#ifndef INVPREF_FTZ_ADAM
-#define INVPREF_FTZ_ADAM 1
-#endif
-#ifndef INVPREF_DIST_SOFTMAX
-#define INVPREF_DIST_SOFTMAX 1
-#endif
-// An extra step of look-ahead with prefetch.global.L2 (no third shared-memory stage needed) was measured and LOSES:
-// user pass 2.91 -> 2.99 ms, re-assignment 3.69 -> 4.66 ms on 25 M samples (round 2, B200): the kernels are bound by
-// DRAM throughput, not by exposed latency, and the prefetches only add request traffic.  Kept as A/B switches.
-// A/B switch (measured, off): user pass, segments with two or more interactions -- request the next segment's stage
-// AFTER the second interaction's item rows instead of at the top of the segment.  cp.async groups complete in order,
-// so the in-loop wait for the item rows (the newest group) also waits for the eight rows of the next stage; ncu's
-// source page shows that wait carrying as many long-scoreboard samples as the top-of-segment wait on half as many
-// executions.  Deferring costs 8 registers (120 -> 128) and measured 2.96-3.01 ms against 2.92 ms (same box).
-#ifndef INVPREF_UPASS_DEFER
-#define INVPREF_UPASS_DEFER 0
-#endif
-// Item pass (ring rows kernel): the six own rows (theta, m, v of both item tables) of a segment are copied global ->
-// shared with cp.async at the top of the segment and read after its interaction loop, instead of being
-// register-destination loads issued before the loop: ptxas attaches the scoreboard wait of such loads to the loop's
-// first branch, and ncu's source page showed 37 % of ALL warp samples of the kernel sitting on that branch.
-// Measured 1.00-1.02 -> 0.95-0.96 ms on C5 (0: the register loads).  Requesting them one segment AHEAD instead (a group
-// of their own, right after the previous segment's rows had been read out of the slots) measured the same 0.95 ms and
-// was not kept.
-#ifndef INVPREF_ITEM_STAGE_OWN
-#define INVPREF_ITEM_STAGE_OWN 1
-#endif
-#ifndef INVPREF_UPASS_L2_PREFETCH
-#define INVPREF_UPASS_L2_PREFETCH 0
-#endif
-#ifndef INVPREF_CLUSTER_L2_PREFETCH
-#define INVPREF_CLUSTER_L2_PREFETCH 0
-#endif
-// Row staging of the re-assignment kernel with cp.async.bulk + mbarrier (UBLKCP / SYNCS) instead of per-lane cp.async
-#ifndef INVPREF_CLUSTER_BULK
-#define INVPREF_CLUSTER_BULK 0
-#endif
-
 namespace invpref {
 
 // One embedding row is handled by a GROUP of 16 lanes; lane l owns NV vectors of VEC floats at
@@ -544,20 +505,12 @@ struct AdamScalars {
 // the fp32 sum, and the reciprocal's argument is >= eps.
 __device__ __forceinline__ float sqrt_approx(float x) {
     float r;
-#if INVPREF_FTZ_ADAM
     asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-#else
-    asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(x));
-#endif
     return r;
 }
 __device__ __forceinline__ float rcp_approx(float x) {
     float r;
-#if INVPREF_FTZ_ADAM
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-#else
-    asm("rcp.approx.f32 %0, %1;" : "=f"(r) : "f"(x));
-#endif
     return r;
 }
 

@@ -18,7 +18,7 @@
 // a fixed order (no floating-point atomics).
 //
 // This file: the staged rows kernel and the launch logic; upass_regs.cu: the chunks kernel and the register-only
-// rows kernel (D > 64, INVPREF_STAGED=0); upass_common.cuh: the per-interaction arithmetic both share.
+// rows kernel (D > 64); upass_common.cuh: the per-interaction arithmetic both share.
 #include "upass_common.cuh"
 
 namespace invpref {
@@ -114,11 +114,7 @@ __global__ void __launch_bounds__(BLOCK, 2) upass_rows_staged_kernel(UserPassArg
     // dataset-scale configs, a few segments per group, the slowest group set the kernel time (18 % of the warp
     // samples sat at the final barrier).  Only the last round can be incomplete, so the first missing segment ends
     // a group's walk.
-#ifdef INVPREF_AB_NOSNAKE
-    auto seg_at = [&](int o) { return o * ng + s0; };
-#else
     auto seg_at = [&](int o) { return o * ng + ((o & 1) ? ng - 1 - s0 : s0); };
-#endif
 
     // prologue: descriptors of the first two segments (the only exposed latency), then group A_0
     request_desc(0, seg_at(0));
@@ -135,41 +131,14 @@ __global__ void __launch_bounds__(BLOCK, 2) upass_rows_staged_kernel(UserPassArg
         const int stg = ord & 1;
         cp_async_wait<0>();      // A_ord: this segment's rows and scalars, the next segment's descriptor
         __syncwarp(gmask);
-        // the next segment's stage (group A_{ord+1}): now -- or, for a segment with more interactions to come, right
-        // after the second interaction's item rows have been requested (INVPREF_UPASS_DEFER, common.cuh)
+        // the next segment's stage (group A_{ord+1}), requested at the top of this one: deferring it until the second
+        // interaction's item rows are requested measured slower (DESIGN.md §3, finding 2)
         auto request_next = [&]() {
             if (seg_at(ord + 1) < n_seg) request_segment(stg ^ 1, meta + UM_DESC + ((ord + 1) & 3) * 8);
             request_desc(ord + 3, seg_at(ord + 3));     // its slot held this group's previous segment
             cp_async_commit();       // A_{ord+1}
         };
-        bool deferred = false;
-#if INVPREF_UPASS_DEFER
-        {
-            const int len0 = meta[UM_DESC + (ord & 3) * 8 + 2] - meta[UM_DESC + (ord & 3) * 8 + 1];
-            deferred = len0 > 1 && len0 <= long_len;
-        }
-#endif
-        if (!deferred) request_next();
-#if INVPREF_UPASS_L2_PREFETCH
-        // One more segment of look-ahead without a third shared-memory stage: the eight rows of segment ord+2 (its
-        // descriptor is already here) are pulled into L2 now, one 128-byte line per lane, so that the cp.async of
-        // group A_{ord+2}, issued one segment from now, pays L2 instead of DRAM latency.
-        if (seg_at(ord + 2) < n_seg) {
-            const int32_t* d2 = meta + UM_DESC + ((ord + 2) & 3) * 8;
-            const int t = lane >> 1, half = lane & 1;
-            const float* tab = a.side.own_inv_in;
-            tab = (t == 1) ? a.side.own_env_in : tab;
-            tab = (t == 2) ? a.side.m_inv : tab;
-            tab = (t == 3) ? a.side.m_env : tab;
-            tab = (t == 4) ? a.side.v_inv : tab;
-            tab = (t == 5) ? a.side.v_env : tab;
-            tab = (t == 6) ? a.side.partner_inv : tab;
-            tab = (t == 7) ? a.side.partner_env : tab;
-            const int64_t r2 = (t >= 6) ? d2[4] : d2[0];
-            if ((EPI == EPI_ADAM || t < 2 || t >= 6) && half * 32 < D)
-                prefetch_l2(tab + r2 * D + half * 32);
-        }
-#endif
+        request_next();
 
         const int4 dA = *reinterpret_cast<const int4*>(meta + UM_DESC + (ord & 3) * 8);       // row, begin, end, n0
         const int4 dB = *reinterpret_cast<const int4*>(meta + UM_DESC + (ord & 3) * 8 + 4);   // p0, n1, p1, -
@@ -224,10 +193,7 @@ __global__ void __launch_bounds__(BLOCK, 2) upass_rows_staged_kernel(UserPassArg
             for (int k = beg; k < end; ++k) {
                 const int par = (k - beg) & 1;
                 if (k > beg) {
-                    // G_{i-1}: this interaction's rows and scalars, the next one's indices.  Deferred stage: it is the
-                    // only group younger than G_0, so the second interaction need not wait for it
-                    if (deferred && k == beg + 1) cp_async_wait<1>();
-                    else cp_async_wait<0>();
+                    cp_async_wait<0>();      // G_{i-1}: this interaction's rows and scalars, the next one's indices
                     __syncwarp(gmask);
                     const int4 sI = *reinterpret_cast<const int4*>(meta + UM_ITS + par * 4);
                     e = sI.x; y = __int_as_float(sI.y); w = __int_as_float(sI.z);
@@ -253,7 +219,6 @@ __global__ void __launch_bounds__(BLOCK, 2) upass_rows_staged_kernel(UserPassArg
                         if (lane == 13) cp_async<4>(smem_addr(meta + UM_ITI + par * 2 + 1), partner + k + 2);
                     }
                     cp_async_commit();       // G_i
-                    if (deferred && k == beg) request_next();
                 }
                 inter_grads<VEC, NV, KT>(a, cfg, myDE, s.sB, rc, rie, q, n, e, y, w, lane, gmask, acc0, Q, ge.x, st, D, K);
                 n = n_a;
@@ -306,20 +271,13 @@ inline size_t upass_ring_bytes(const Geometry& g) {   // staged rows + per-group
 inline size_t upass_ring_offset(const Geometry& g) {   // bytes before the ring: the carve of upass_smem, 128-byte aligned
     return (size_t)ring_align_up((4 + 2 * GROUPS_PER_BLOCK) * g.K * g.D + SB_WORDS) * sizeof(float);
 }
-inline bool upass_staged(const Geometry& g) {
-    static const bool enabled = [] {
-        const char* e = getenv("INVPREF_STAGED");   // INVPREF_STAGED=0: register-only rows kernel (A/B runs)
-        return !(e && e[0] == '0');
-    }();
-    return enabled && g.NV * g.VEC <= 4;
-}
 
 }  // namespace
 
 bool upass_supported(const Geometry& g) { return upass_smem(g) <= 96 * 1024; }
 
 static bool use_staged(const Geometry& g) {
-    return upass_staged(g) && upass_ring_offset(g) + upass_ring_bytes(g) <= 227 * 1024;
+    return g.NV * g.VEC <= 4 && upass_ring_offset(g) + upass_ring_bytes(g) <= 227 * 1024;
 }
 
 int upass_rows_grid(const Geometry& g, int64_t max_seg) {

@@ -86,7 +86,7 @@ __device__ __forceinline__ void inter_grads(const UserPassArgs& a, const LossCfg
     for (int kk = 0; kk < KT; ++kk) lg[kk] = (kk < K) ? group_sum(q.lg[kk], gmask) + sB[kk] : -INFINITY;
 
     float g_z1, g_z2, gl[KT], lw[3];
-    loss_grads<KT, INVPREF_DIST_SOFTMAX != 0>(cfg, z1, z2, lg, y, w, e, g_z1, g_z2, gl, lw, lane, gmask);
+    loss_grads<KT, true>(cfg, z1, z2, lg, y, w, e, g_z1, g_z2, gl, lw, lane, gmask);
     st.sq += q.sq;
     st.ab += q.ab;
     {
@@ -122,11 +122,7 @@ __device__ __forceinline__ void inter_grads(const UserPassArgs& a, const LossCfg
         out[0] = g_z1;
         out[1] = g_z2;
         out[2] = __int_as_float(e);
-#ifdef INVPREF_AB_NOSB
-        const float neg_alpha = a.neg_alpha;
-#else
         const float neg_alpha = sB[SB_NEG_ALPHA];
-#endif
 #pragma unroll
         for (int kk = 0; kk < 9; ++kk) out[3 + kk] = (kk < KT) ? neg_alpha * gl[kk < KT ? kk : 0] : 0.f;
         *reinterpret_cast<float4*>(gp) = make_float4(out[0], out[1], out[2], out[3]);
@@ -168,11 +164,7 @@ __device__ __forceinline__ void finish_range(const UserPassArgs& a, const float*
                                              float* __restrict__ myDW, const Row<VEC, NV>& ra, int lane,
                                              const float (&acc0)[NV * VEC], const float (&Q)[KT][NV * VEC],
                                              Row<VEC, NV>& gi, int D, int K, const float* __restrict__ sB) {
-#ifdef INVPREF_AB_NOSB
-    const float neg_alpha = a.neg_alpha;
-#else
     const float neg_alpha = sB[SB_NEG_ALPHA];
-#endif
 #pragma unroll
     for (int j = 0; j < NV; ++j) {
         const int d0 = dim_of<VEC>(lane, j);
@@ -221,10 +213,8 @@ struct Smem {
 };
 
 __device__ __forceinline__ AdamScalars adam_from_smem(AdamScalars s, const float* sB) {
-#ifndef INVPREF_AB_NOSB
     s.step_size = sB[SB_STEP_SIZE];
     s.inv_bc2_sqrt = sB[SB_INV_BC2];
-#endif
     return s;
 }
 

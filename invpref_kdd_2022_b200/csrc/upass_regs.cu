@@ -1,6 +1,6 @@
 // Fused user pass, register-only kernels: upass_chunks_kernel (CHUNK-sized pieces of long user segments, for
 // every geometry) and upass_rows_kernel (every user segment; used for row slices wider than 16 bytes per lane,
-// i.e. D > 64, and with INVPREF_STAGED=0 for A/B runs).  See upass.cu for the staged rows kernel.
+// i.e. D > 64).  See upass.cu for the staged rows kernel.
 #include "upass_common.cuh"
 
 namespace invpref {
@@ -214,7 +214,9 @@ int launch_upass_rows_regs(const Geometry& g, const UserPassArgs& a, int epi, in
         else if (epi == EPI_ADAM) LAUNCH((upass_rows_kernel<V, N, KT_, EPI_ADAM, false>));                       \
         else LAUNCH((upass_rows_kernel<V, N, KT_, EPI_EXPORT, false>));                                          \
     } while (0)
-    INVPREF_DISPATCH_GEOM(g, CALL);
+    // every narrower row slice takes the staged kernel (use_staged, upass.cu): only VEC = 4 with NV = 2 or 4 get here
+    if (g.NV == 2) INVPREF_DISPATCH_K(4, 2, g.KT, CALL);
+    else INVPREF_DISPATCH_K(4, 4, g.KT, CALL);
 #undef CALL
 #undef LAUNCH
     count_launch();

@@ -54,7 +54,7 @@ class HotPath:
         self._ws_batch = -1
         self.loss_buf = torch.zeros(6, dtype=torch.float32, device=self.device)
         # lazy Adam needs the fused user pass; shapes that only have the unfused path (K * D too large for the
-        # per-CTA dE/dW slices, or INVPREF_FUSED=0) run plain dense Adam -- same results, more HBM traffic
+        # per-CTA dE/dW slices) run plain dense Adam -- same results, more HBM traffic
         self.lazy_supported = self.lib.invpref_upass_supported(C.byref(self.desc)) == 1
         self.lazy_requested = bool(lazy)
         self.lazy = bool(lazy) and self.lazy_supported
