@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define INVPREF_ABI_VERSION 2
+#define INVPREF_ABI_VERSION 3
 #define INVPREF_MAX_ENVS 8      /* drivers use K = 2, 4, 5, 6 */
 #define INVPREF_MAX_DIM 256     /* drivers use D = 30, 40; synthetic config D = 64 */
 #define INVPREF_NUM_LOSSES 6    /* train.py:836-843: invariant, env_aware, envs, L2, L1, loss */
@@ -335,34 +335,27 @@ int invpref_eval_topk(const invpref_desc* desc, const invpref_params* params, co
                       const int64_t* pool_items, const int64_t* gt_off, const int64_t* gt_items, int32_t k,
                       int64_t* top_items, float* top_scores, uint8_t* hits, int64_t* n_gt, void* stream);
 
-/* ---- the same exchange over peer memory (NVLink loads; no collective on the data path) -------------
- * `tables` / `grads`: HOST arrays of 2 * world device pointers, [t * world + rank] = base of item table t
- * (0 invariant, 1 env-aware) / of the partial-gradient cache t of rank `rank`, the caller's own rank
- * included; the peers' buffers must be mapped into this process (CUDA IPC / VMM, e.g. torch symmetric
- * memory).  The caller orders producers and consumers across ranks with a barrier.
+/* ---- the same exchange over peer memory (no collective on the data path) ------------------------------------
+ * Pointer arrays are HOST arrays of device pointers into the ranks' buffers, the caller's own rank included; the
+ * peers' buffers must be mapped into this process (CUDA IPC / VMM, e.g. torch symmetric memory).  The caller orders
+ * producers and consumers across ranks with a barrier.
  *
- * invpref_fetch_rows_p2p: out_t[c, :] = tables[t * world + owner[c]][rows[c], :] for c < n, t = 0, 1
- * (replaces invpref_gather_rows on the owners + an all-to-all of rows). */
+ * invpref_fetch_rows_p2p: out_t[c, :] = tables[t * world + owner[c]][rows[c], :] for c < n, t = 0, 1, where
+ * tables[t * world + rank] = base of item table t (0 invariant, 1 env-aware) of rank `rank` (NVLink loads; replaces
+ * invpref_gather_rows on the owners + an all-to-all of rows). */
 int invpref_fetch_rows_p2p(const float* const* tables, int32_t world, const int32_t* owner, const int64_t* rows,
                            int64_t n, int32_t dim, float* out_inv, float* out_env, void* stream);
 
-/* invpref_owner_adam_p2p: for every row j < n_rows of the caller's item shard and t = 0, 1:
- * g = sum over ranks p = 0..world-1 (in this order) of grads[t * world + p][pos[p * n_rows + j], :]
- * (pos < 0: rank p has no partial for row j), then one dense torch.optim.Adam step on theta/m/v with g --
- * the same order and arithmetic as zero-fill + invpref_scatter_add_rows per rank + invpref_adam_dense, in one
- * kernel reading the partials where the ranks' item passes wrote them. */
-int invpref_owner_adam_p2p(float* theta_inv, float* theta_env, float* m_inv, float* m_env, float* v_inv, float* v_env,
-                           int64_t n_rows, int32_t dim, int32_t world, const float* const* grads, const int32_t* pos,
-                           const invpref_hyper* hyper, void* stream);
-
-/* invpref_owner_adam_push: the push counterpart of invpref_owner_adam_p2p, reading LOCAL memory and writing peers.
+/* invpref_owner_adam_push: the owner's side of the push exchange, reading LOCAL memory and writing peers.
  * For every row j < n_rows of the caller's item shard and t = 0, 1:
  *   g = sum over ranks p = 0..world-1 (in this order) of stage_t[spos[p * n_rows + j], :]   (spos < 0: no partial)
- *   one dense torch.optim.Adam step on theta/m/v with g  (same order and arithmetic as invpref_owner_adam_p2p), then
+ *   one dense torch.optim.Adam step on theta/m/v with g, then
  *   for every rank p with npos[p * n_rows + j] >= 0: caches[t * world + p][npos[p * n_rows + j], :] = updated row
- * i.e. the updated row is pushed into the slot it has in rank p's row cache for the NEXT batch (posted NVLink
- * writes; replaces invpref_fetch_rows_p2p).  stage_*: the caller's own staging buffers, filled by the ranks' item
- * passes (invpref_push).  caches: HOST array of 2 * world device pointers; npos / caches may be NULL (last batch). */
+ * The sum and the Adam step have the order and arithmetic of the collective path: zero-fill, then
+ * invpref_scatter_add_rows of each rank's partials in rank order, then invpref_adam_dense.  The updated row is pushed
+ * into the slot it has in rank p's row cache for the NEXT batch (posted NVLink writes; replaces
+ * invpref_fetch_rows_p2p).  stage_*: the caller's own staging buffers, filled by the ranks' item passes
+ * (invpref_push).  caches: HOST array of 2 * world device pointers; npos / caches may be NULL (last batch). */
 int invpref_owner_adam_push(float* theta_inv, float* theta_env, float* m_inv, float* m_env, float* v_inv, float* v_env,
                             int64_t n_rows, int32_t dim, int32_t world, const float* stage_inv, const float* stage_env,
                             const int32_t* spos, float* const* caches, const int32_t* npos,

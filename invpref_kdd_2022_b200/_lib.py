@@ -25,7 +25,7 @@ EXPORTS = (
     "invpref_backward", "invpref_train_step", "invpref_cluster", "invpref_stat_envs",
     "invpref_env_hist", "invpref_launch_count", "invpref_profile_enable", "invpref_profile_steps",
     "invpref_profile_read", "invpref_adam_dense", "invpref_gather_rows", "invpref_scatter_add_rows",
-    "invpref_user_sweep", "invpref_flush_users", "invpref_fetch_rows_p2p", "invpref_owner_adam_p2p",
+    "invpref_user_sweep", "invpref_flush_users", "invpref_fetch_rows_p2p",
     "invpref_mask_scores", "invpref_hits_from_csr", "invpref_upass_supported", "invpref_plan_status",
     "invpref_check_ids", "invpref_dyn_fill", "invpref_graph_begin", "invpref_graph_end", "invpref_graph_launch",
     "invpref_graph_destroy", "invpref_graph_launches", "invpref_owner_adam_push", "invpref_eval_topk",
@@ -129,8 +129,6 @@ def load() -> C.CDLL:
     lib.invpref_gather_rows.argtypes = [vp, vp, i64, C.c_int32, vp, vp]
     lib.invpref_scatter_add_rows.argtypes = [vp, vp, i64, C.c_int32, vp, vp]
     lib.invpref_fetch_rows_p2p.argtypes = [C.POINTER(vp), C.c_int32, vp, vp, i64, C.c_int32, vp, vp, vp]
-    lib.invpref_owner_adam_p2p.argtypes = [vp, vp, vp, vp, vp, vp, i64, C.c_int32, C.c_int32, C.POINTER(vp), vp,
-                                           C.POINTER(Hyper), vp]
     lib.invpref_owner_adam_push.argtypes = [vp, vp, vp, vp, vp, vp, i64, C.c_int32, C.c_int32, vp, vp, vp,
                                             C.POINTER(vp), vp, C.POINTER(Hyper), vp]
     lib.invpref_peer_allreduce.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(vp), C.POINTER(vp),
@@ -154,7 +152,7 @@ def load() -> C.CDLL:
     return lib
 
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 ERR_ID_RANGE = -7
 
 

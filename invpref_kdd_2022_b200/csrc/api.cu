@@ -553,18 +553,6 @@ int invpref_fetch_rows_p2p(const float* const* tables, int32_t world, const int3
     return launch_fetch_rows_p2p(tables, world, owner, rows, n, dim, out_inv, out_env, (cudaStream_t)stream);
 }
 
-int invpref_owner_adam_p2p(float* theta_inv, float* theta_env, float* m_inv, float* m_env, float* v_inv, float* v_env,
-                           int64_t n_rows, int32_t dim, int32_t world, const float* const* grads, const int32_t* pos,
-                           const invpref_hyper* hyper, void* stream) {
-    if (n_rows < 0 || dim < 1 || !grads || !hyper || hyper->step < 1) return INVPREF_ERR_BAD_ARG;
-    if (n_rows > 0 && (!theta_inv || !theta_env || !m_inv || !m_env || !v_inv || !v_env || !pos)) return INVPREF_ERR_BAD_ARG;
-    for (int i = 0; i < 2 * world && world >= 1 && world <= 16; ++i)
-        if (!grads[i]) return INVPREF_ERR_BAD_ARG;
-    if (n_rows == 0) return INVPREF_OK;
-    return launch_owner_adam_p2p(theta_inv, theta_env, m_inv, m_env, v_inv, v_env, n_rows, dim, world, grads, pos,
-                                 make_adam(hyper), hyper->dyn, (cudaStream_t)stream);
-}
-
 int invpref_owner_adam_push(float* theta_inv, float* theta_env, float* m_inv, float* m_env, float* v_inv, float* v_env,
                             int64_t n_rows, int32_t dim, int32_t world, const float* stage_inv, const float* stage_env,
                             const int32_t* spos, float* const* caches, const int32_t* npos,

@@ -6,14 +6,15 @@
 //  scatter_add_rows_kernel : adds one peer's partial row gradients into the owner's shard; indices are
 //                            unique within a call, peers are applied in rank order => deterministic.
 //
-// Over peer memory (NVLink loads from the other ranks' buffers, mapped into this process -- e.g. torch
-// symmetric memory; no NCCL on the data path, the caller only needs a barrier between producers and consumers):
-//  fetch_rows_p2p_kernel   : cache[c] = table_of(owner[c])[rows[c]] for both item tables: replaces
+// Over peer memory (the other ranks' buffers, mapped into this process -- e.g. torch symmetric memory; no NCCL on
+// the data path, the caller only needs a barrier between producers and consumers):
+//  fetch_rows_p2p_kernel   : cache[c] = table_of(owner[c])[rows[c]] for both item tables (NVLink loads): replaces
 //                            gather_rows + all-to-all of rows.
-//  owner_adam_p2p_kernel   : for every row of the owner's shard, the partial gradients are read straight from
-//                            the ranks' gradient caches, summed in rank order (same order and arithmetic as
-//                            zero + scatter_add per rank) and consumed by Adam in registers: replaces the
-//                            all-to-all of gradients + zero-fill + G scatter-adds + adam_dense.
+//  owner_adam_push_kernel  : for every row of the owner's shard, the partial gradients the ranks' item passes
+//                            stored into its staging are summed in rank order (same order and arithmetic as
+//                            zero-fill + scatter_add per rank) and consumed by Adam in registers; the updated row is
+//                            stored into the requesters' caches (NVLink stores): replaces the all-to-all of
+//                            gradients + zero-fill + G scatter-adds + adam_dense + the next batch's row exchange.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -117,64 +118,12 @@ __global__ void __launch_bounds__(256) fetch_rows_p2p_kernel(PeerPtrs tables, in
     }
 }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) owner_adam_p2p_kernel(float* __restrict__ th0, float* __restrict__ th1,
-                                                             float* __restrict__ m0, float* __restrict__ m1,
-                                                             float* __restrict__ v0, float* __restrict__ v1,
-                                                             int64_t n_rows, int dim, int world, PeerPtrs grads,
-                                                             const int32_t* __restrict__ pos, AdamScalars s0,
-                                                             const invpref_dyn* dyn) {
-    const AdamScalars s = with_dyn(s0, dyn);
-    const int per_row = dim / VEC;
-    const int64_t per_table = n_rows * per_row, total = 2 * per_table;
-    for (int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < total; q += (int64_t)gridDim.x * blockDim.x) {
-        const int t = q >= per_table ? 1 : 0;
-        const int64_t rem = q - t * per_table;
-        const int64_t j = (int64_t)((uint32_t)rem / (uint32_t)per_row);   // per_table < 2^31 (checked at launch)
-        const int c = (int)(rem - j * per_row) * VEC;
-        // all slots first, then all (independent) remote loads, then the sum in rank order
-        int sl[P2P_MAX_WORLD];
-        float part[P2P_MAX_WORLD][VEC];
-#pragma unroll
-        for (int p = 0; p < P2P_MAX_WORLD; ++p) sl[p] = (p < world) ? pos[(int64_t)p * n_rows + j] : -1;
-#pragma unroll
-        for (int p = 0; p < P2P_MAX_WORLD; ++p) {
-            if (sl[p] >= 0) {
-                ldv_sys<VEC>(grads.p[t * world + p] + (int64_t)sl[p] * dim + c, part[p]);
-            } else {
-#pragma unroll
-                for (int x = 0; x < VEC; ++x) part[p][x] = 0.f;
-            }
-        }
-        float g[VEC];
-#pragma unroll
-        for (int x = 0; x < VEC; ++x) g[x] = 0.f;
-#pragma unroll
-        for (int p = 0; p < P2P_MAX_WORLD; ++p)
-            if (sl[p] >= 0) {
-#pragma unroll
-                for (int x = 0; x < VEC; ++x) g[x] += part[p][x];
-            }
-        float* th = (t ? th1 : th0) + j * dim + c;
-        float* mm = (t ? m1 : m0) + j * dim + c;
-        float* vv = (t ? v1 : v0) + j * dim + c;
-        float pr[VEC], mr[VEC], vr[VEC];
-        ldv_stream<VEC>(th, pr);
-        ldv_stream<VEC>(mm, mr);
-        ldv_stream<VEC>(vv, vr);
-#pragma unroll
-        for (int x = 0; x < VEC; ++x) adam_update(pr[x], mr[x], vr[x], g[x], s);
-        stv<VEC>(th, pr);
-        stv_stream<VEC>(mm, mr);
-        stv_stream<VEC>(vv, vr);
-    }
-}
-
 struct PeerOut { float* p[2 * P2P_MAX_WORLD]; };
 
 // Owner side of the PUSH exchange: partials from LOCAL staging (the ranks' item passes stored them there over
 // NVLink), summed in rank order, Adam in registers, and the updated row stored into every requester's row cache
-// for the next batch (posted NVLink writes).  Same per-element arithmetic and order as owner_adam_p2p_kernel.
+// for the next batch (posted NVLink writes).  Same per-element arithmetic and order as the collective path: zero-fill,
+// scatter_add_rows_kernel per rank in rank order, adam_dense_kernel.
 // WMAX: compile-time bound of the rank loops (2, 4, 8, 16): the position loads, the staging loads and the pushes are
 // fully unrolled and all in flight together.
 template <int VEC, int WMAX>
@@ -349,20 +298,6 @@ int launch_fetch_rows_p2p(const float* const* tables_host, int world, const int3
     for (int i = 0; i < 2 * world; ++i) { pp.p[i] = tables_host[i]; v4 = v4 && ((uintptr_t)tables_host[i] % 16 == 0); }
     if (v4) fetch_rows_p2p_kernel<4><<<grid_1d(2 * n * (dim / 4) / 4 + 256), 256, 0, stream>>>(pp, world, owner, rows, n, dim, out0, out1);
     else fetch_rows_p2p_kernel<1><<<grid_1d(2 * n * dim / 4 + 256), 256, 0, stream>>>(pp, world, owner, rows, n, dim, out0, out1);
-    count_launch();
-    return cudaGetLastError() == cudaSuccess ? INVPREF_OK : INVPREF_ERR_CUDA;
-}
-
-int launch_owner_adam_p2p(float* th0, float* th1, float* m0, float* m1, float* v0, float* v1, int64_t n_rows, int dim,
-                          int world, const float* const* grads_host, const int32_t* pos, const AdamScalars& s,
-                          const invpref_dyn* dyn, cudaStream_t stream) {
-    if (world < 1 || world > P2P_MAX_WORLD || n_rows * (int64_t)dim >= 0x7fffffffLL) return INVPREF_ERR_BAD_ARG;
-    PeerPtrs pp = {};
-    bool v4 = dim % 4 == 0;
-    for (float* q : {th0, th1, m0, m1, v0, v1}) v4 = v4 && ((uintptr_t)q % 16 == 0);
-    for (int i = 0; i < 2 * world; ++i) { pp.p[i] = grads_host[i]; v4 = v4 && ((uintptr_t)grads_host[i] % 16 == 0); }
-    if (v4) owner_adam_p2p_kernel<4><<<grid_1d(2 * n_rows * (dim / 4)), 256, 0, stream>>>(th0, th1, m0, m1, v0, v1, n_rows, dim, world, pp, pos, s, dyn);
-    else owner_adam_p2p_kernel<1><<<grid_1d(2 * n_rows * dim), 256, 0, stream>>>(th0, th1, m0, m1, v0, v1, n_rows, dim, world, pp, pos, s, dyn);
     count_launch();
     return cudaGetLastError() == cudaSuccess ? INVPREF_OK : INVPREF_ERR_CUDA;
 }

@@ -148,9 +148,6 @@ int launch_scatter_add_rows(const float* src, const int64_t* rows, int64_t n, in
 // peer-memory variants (pointer arrays are HOST arrays of 2 * world device pointers: [t * world + rank])
 int launch_fetch_rows_p2p(const float* const* tables_host, int world, const int32_t* owner, const int64_t* rows,
                           int64_t n, int dim, float* out0, float* out1, cudaStream_t stream);
-int launch_owner_adam_p2p(float* th0, float* th1, float* m0, float* m1, float* v0, float* v1, int64_t n_rows, int dim,
-                          int world, const float* const* grads_host, const int32_t* pos, const AdamScalars& s,
-                          const invpref_dyn* dyn, cudaStream_t stream);
 int launch_owner_adam_push(float* th0, float* th1, float* m0, float* m1, float* v0, float* v1, int64_t n_rows, int dim,
                            int world, const float* stage0, const float* stage1, const int32_t* spos,
                            float* const* caches_host, const int32_t* npos, const AdamScalars& s,

@@ -6,7 +6,7 @@ ranks; value = K * global_batch / that time.
 
 Legs of the one JSON line rank 0 prints:
   headline        C5 (10 M x 1 M, D 64, B 2^22), users + items row-sharded, item exchange over peer memory
-                  (INVPREF_EXCHANGE = push (default) | pull | nccl);
+                  (INVPREF_EXCHANGE = push (default) | nccl);
   parity_vs_1gpu  a reduced shape trained for a few steps by the N ranks (same exchange) AND by rank 0 alone: losses
                   and every gathered table compared (tolerance: the summation order of the item partials differs), plus
                   bit-equality of the peer-memory exchange with the NCCL all-to-all exchange on the real ranks;
@@ -24,63 +24,48 @@ import torch.distributed as dist
 
 
 def _exchange_mode():
-    m = os.environ.get("INVPREF_EXCHANGE", "").lower()
-    if m in ("push", "pull", "nccl"):
-        return m
-    return "nccl" if os.environ.get("INVPREF_P2P", "1") == "0" else "push"
+    m = (os.environ.get("INVPREF_EXCHANGE") or "push").lower()
+    if m not in ("push", "nccl"):
+        raise ValueError(f"INVPREF_EXCHANGE must be 'push' or 'nccl', not {m!r}")
+    return m
 
 
 def make_sharded(w, U, I, Bg, rank, world, dev, mode, init=None, lazy=True, sync=None):
-    """A ShardedTrainer wired for `mode`; falls back (all ranks together) to the NCCL exchange if symmetric memory
-    is unavailable.  Returns (trainer, note)."""
+    """A ShardedTrainer wired for `mode` ("push" or "nccl"); falls back (all ranks together) to the NCCL exchange if
+    symmetric memory is unavailable.  Returns (trainer, note, mode)."""
     from invpref_kdd_2022_b200.parallel import ShardedTrainer, SymmetricItemStorage
     K, D = w["K"], w["D"]
     cache_rows = min(I, Bg // world * 2 + 1024)
-    stage_rows = min(2 * cache_rows, (I + world - 1) // world * world) if mode == "push" else 0
+    stage_rows = min(2 * cache_rows, (I + world - 1) // world * world)
     store, why = None, "disabled (INVPREF_EXCHANGE=nccl)"
     peer_sync = os.environ.get("INVPREF_SYNC", "peer").lower() != "nccl" if sync is None else bool(sync)
     n_small = 2 * K * D + K + 6
-    if mode != "nccl":
+    if mode == "push":
         try:
             store = SymmetricItemStorage(I, D, world, cache_rows, dev, dist.group.WORLD, stage_rows=stage_rows,
                                          sync_floats=n_small if peer_sync else 0)
             why = ""
         except Exception as ex:      # noqa: BLE001 -- any failure means "use NCCL"
             store, why = None, f"{type(ex).__name__}: {ex}"[:200]
-    sync_store = None
-    if mode == "nccl" and sync:      # NCCL row / gradient exchange, but the step's all-reduce + barriers over peer memory
-        try:                         # (parity_check: isolates the exchange path, same summation order of E / W / b)
-            sync_store = SymmetricItemStorage(world, D, world, 1, dev, dist.group.WORLD, sync_floats=n_small)
+    elif sync:      # NCCL row / gradient exchange, but the step's all-reduce + barriers over peer memory
+        try:        # (parity_check: isolates the exchange path, same summation order of E / W / b)
+            store = SymmetricItemStorage(I, D, world, cache_rows, dev, dist.group.WORLD, sync_floats=n_small)
         except Exception:            # noqa: BLE001
-            sync_store = None
-    ok = torch.tensor([1 if (store is not None or mode == "nccl") else 0,
-                       1 if (sync_store is not None or not (mode == "nccl" and sync)) else 0], device=dev)
+            store = None
+    ok = torch.tensor([1 if (store is not None or not (mode == "push" or sync)) else 0], device=dev)
     dist.all_reduce(ok, op=dist.ReduceOp.MIN)
-    if int(ok[0].item()) == 0:
+    if int(ok.item()) == 0:
         store, mode = None, "nccl"
-    if int(ok[1].item()) == 0:
-        sync_store = None
     tr = ShardedTrainer(U, I, K, D, w["implicit"], w["roe"], w["ree"], w["lr"], rank, world, dev,
-                        cache_rows=cache_rows, alloc=store.alloc if store is not None else None, init=init, lazy=lazy,
-                        stage_rows=stage_rows if store is not None else 0)
-    if store is not None:
-        tr.enable_p2p(store.ptrs("Iinv"), store.ptrs("Ienv"), store.ptrs("gcache0"), store.ptrs("gcache1"))
-        note = "peer memory (torch symmetric memory), NVLink pulls"
-        if mode == "push":
-            tr.enable_push([[store.ptrs(f"stage{par}{t}") for t in range(2)] for par in range(2)],
-                           [store.ptrs(f"cache{t}") for t in range(2)])
-            note = "peer memory (torch symmetric memory): item pass pushes partial gradients into the owners' " \
-                   "staging, owners push updated rows into the requesters' next-batch caches (posted NVLink writes)"
-        if peer_sync:
-            tr.enable_peer_sync(store.ptrs("sync_slots"), store.ptrs("sync_flags"), store.sync_floats)
+                        cache_rows=cache_rows, init=init, lazy=lazy, store=store)
+    if tr.push is not None:
+        note = "peer memory (torch symmetric memory): item pass pushes partial gradients into the owners' " \
+               "staging, owners push updated rows into the requesters' next-batch caches (posted NVLink writes)"
+        if tr.sync is not None:
             note += "; E/W/b gradient all-reduce and both step barriers over peer memory too (invpref_peer_allreduce: " \
                     "no NCCL call in the step)"
-        tr._store = store
     else:
         note = "NCCL all-to-all (" + (why or "a peer could not map symmetric memory") + ")"
-        if sync_store is not None:
-            tr.enable_peer_sync(sync_store.ptrs("sync_slots"), sync_store.ptrs("sync_flags"), sync_store.sync_floats)
-            tr._store = sync_store
     torch.cuda.synchronize()
     dist.barrier()                       # every shard initialised before anyone touches a peer's memory
     return tr, note, mode

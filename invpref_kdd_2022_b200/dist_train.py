@@ -50,8 +50,8 @@ class _ShardedInvPrefTrainManager:
         (models.py:415-418): the sharded tables live in this object, not in an ``nn.Module``.  ``training_data``:
         int64 ``[n, 3]`` (user, item, score) -- the whole training set, or, with ``local_rows`` (their global row
         numbers, ascending) and ``total_rows``, only the rows whose user this rank owns.  ``init``: optional full
-        tables (tests).  ``exchange``: "push" | "pull" (peer memory, needs torch symmetric memory) | "nccl".
-        ``peer_sync``: with a peer-memory exchange, also run the step's small all-reduce and barriers over peer
+        tables (tests).  ``exchange``: "push" (peer memory, needs torch symmetric memory) | "nccl".
+        ``peer_sync``: with the push exchange, also run the step's small all-reduce and barriers over peer
         memory (``invpref_peer_allreduce``) instead of NCCL.  ``use_graph``: with push + peer_sync (a step is then
         nothing but library kernels) every epoch after the first is replayed as ONE CUDA-graph launch per rank.
         ``driver`` / ``rank`` / ``world``: for simulated ranks (tests); default: torch.distributed.
@@ -59,6 +59,8 @@ class _ShardedInvPrefTrainManager:
         the host, "numpy_device" draws the same values on the GPU (npstream.py), one global batch at a time."""
         if tie_break_rng not in ("numpy", "numpy_device"):
             raise ValueError("tie_break_rng must be 'numpy' or 'numpy_device'")
+        if exchange not in ("push", "nccl"):
+            raise ValueError("exchange must be 'push' or 'nccl'")
         self.tie_break_rng = tie_break_rng
         if driver is None and world == 1:
             from .parallel import LocalDriver
@@ -126,28 +128,17 @@ class _ShardedInvPrefTrainManager:
         stage_rows = min(2 * cache_rows + 1024, ((item_num + self.world - 1) // self.world) * self.world) \
             if exchange == "push" else 0
         self.exchange = exchange
-        self._store = None
-        alloc = None
-        if exchange in ("push", "pull") and driver is None:
+        store = None
+        if exchange == "push" and driver is None:
             from .parallel import SymmetricItemStorage
             import torch.distributed as dist
-            self._store = SymmetricItemStorage(item_num, factor_num, self.world, cache_rows, device,
-                                               group if group is not None else dist.group.WORLD,
-                                               stage_rows=stage_rows,
-                                               sync_floats=(2 * env_num * factor_num + env_num + 6) if peer_sync else 0)
-            alloc = self._store.alloc
+            store = SymmetricItemStorage(item_num, factor_num, self.world, cache_rows, device,
+                                         group if group is not None else dist.group.WORLD, stage_rows=stage_rows,
+                                         sync_floats=(2 * env_num * factor_num + env_num + 6) if peer_sync else 0)
         self.trainer = ShardedTrainer(user_num, item_num, env_num, factor_num, self.implicit, reg_only_embed,
                                       reg_env_embed, lr, self.rank, self.world, device, cache_rows=cache_rows, init=init,
-                                      seed=seed, lazy=lazy_adam, alloc=alloc, stage_rows=stage_rows)
-        if self._store is not None:
-            st = self._store
-            self.trainer.enable_p2p(st.ptrs("Iinv"), st.ptrs("Ienv"), st.ptrs("gcache0"), st.ptrs("gcache1"))
-            if exchange == "push":
-                self.trainer.enable_push([[st.ptrs(f"stage{par}{t}") for t in range(2)] for par in range(2)],
-                                         [st.ptrs(f"cache{t}") for t in range(2)])
-            if peer_sync:
-                self.trainer.enable_peer_sync(st.ptrs("sync_slots"), st.ptrs("sync_flags"), st.sync_floats)
-            import torch.distributed as dist
+                                      seed=seed, lazy=lazy_adam, store=store, stage_rows=stage_rows)
+        if store is not None:
             torch.cuda.synchronize()
             dist.barrier(group)
         self.engine = self.trainer.hot
@@ -281,10 +272,10 @@ class _ShardedInvPrefTrainManager:
         self._prepare()
         tr = self.trainer
         tr.flush()
-        if self._store is not None:
+        if tr.store is not None:
             import torch.distributed as dist
             torch.cuda.synchronize()
-            dist.barrier(self.group)          # every owner's rows are final before anyone pulls them
+            dist.barrier(self.group)          # every owner's rows are final before anyone fetches them
         new_envs = torch.empty_like(self.envs)
         acc = torch.zeros(self.envs_num + 1, dtype=torch.int64, device=self.device)
         for b, sb in enumerate(self._batches):

@@ -214,14 +214,14 @@ class ItemRoute:
         self.recv_splits = None    # list[G]     cache rows coming from each owner
         self.send_splits = None    # list[G]     rows of my shard going to each requester
         self.send_rows = None      # int64 [sum(send_splits)] owner-local row indices, grouped by requester
-        # peer-memory exchange (ShardedTrainer.enable_p2p)
+        # push exchange over peer memory (ShardedTrainer.enable_push).  Rows: a requester loads cache slot c from
+        # owner slot_owner[c]'s shard (first fetch), and owners store their updated rows into the requesters' caches
+        # at pos.  Gradients: owners keep a staging buffer laid out like send_rows (grouped by requester); a
+        # requester stores the partial gradient of cache slot c into owner slot_owner[c]'s staging at push_index[c]
         self.slot_owner = None     # int32 [n_cache] owner rank of every cache slot
         self.want_rows = None      # int64 [n_cache] owner-local row of every cache slot
         self.peer_first = None     # list[G]     first slot, in requester p's cache, of the rows it wants from me
-        self.pos = None            # int32 [G, I_loc] slot of my row j in rank p's (gradient / row) cache, or -1
-        # push exchange (ShardedTrainer.enable_push): owners keep a staging buffer laid out like send_rows (grouped
-        # by requester); a requester stores the partial gradient of cache slot c into owner slot_owner[c]'s staging
-        # at push_index[c]
+        self.pos = None            # int32 [G, I_loc] slot of my row j in rank p's row cache, or -1
         self.peer_off = None       # list[G]     first staging row, at owner o, of the block of rows I want from o
         self.push_index = None     # int32 [n_cache] row in the owner's staging buffer of every cache slot
         self.spos = None           # int32 [G, I_loc] row in MY staging buffer of rank p's partial for my row j, or -1
@@ -265,53 +265,45 @@ def build_route_gen(items_global: torch.Tensor, world: int, route: ItemRoute):
     return route
 
 
-def build_pos_table(route: ItemRoute, world: int, n_local_rows: int) -> torch.Tensor:
-    """pos[p, j] = slot of my item row j in rank p's gradient cache, -1 if rank p did not ask for it."""
+def build_slot_table(route: ItemRoute, world: int, n_local_rows: int, first) -> torch.Tensor:
+    """t[p, j] = first[p] + k if my item row j is the k-th row rank p asked me for, -1 if rank p did not ask for it.
+    ``first = route.peer_first``: the slot of row j in rank p's row cache (route.pos).  ``first[p] =
+    sum(send_splits[:p])``: the row of my staging buffer, laid out like send_rows, that holds rank p's partial gradient
+    of row j (route.spos)."""
     dev = route.send_rows.device
-    pos = torch.full((world, max(n_local_rows, 1)), -1, dtype=torch.int32, device=dev)
+    tab = torch.full((world, max(n_local_rows, 1)), -1, dtype=torch.int32, device=dev)
     o = 0
     for p in range(world):
         n = route.send_splits[p]
         if n:
-            pos[p, route.send_rows[o:o + n]] = (route.peer_first[p] + torch.arange(n, device=dev)).to(torch.int32)
+            tab[p, route.send_rows[o:o + n]] = (first[p] + torch.arange(n, device=dev)).to(torch.int32)
         o += n
-    return pos
-
-
-def build_spos_table(route: ItemRoute, world: int, n_local_rows: int) -> torch.Tensor:
-    """spos[p, j] = row, in MY staging buffer, where rank p's item pass stores its partial gradient of my item row
-    j (-1: rank p has none).  The staging buffer is laid out like send_rows: grouped by requester, in its order."""
-    dev = route.send_rows.device
-    spos = torch.full((world, max(n_local_rows, 1)), -1, dtype=torch.int32, device=dev)
-    o = 0
-    for p in range(world):
-        n = route.send_splits[p]
-        if n:
-            spos[p, route.send_rows[o:o + n]] = (o + torch.arange(n, device=dev)).to(torch.int32)
-        o += n
-    return spos
+    return tab
 
 
 class SymmetricItemStorage:
-    """Peer-visible storage of one rank's item shard and partial-gradient caches: ONE torch symmetric-memory
-    buffer [Iinv | Ienv | gcache0 | gcache1] with the same layout on every rank, so that a peer's table is
-    `buffer_ptrs[rank] + offset`.  Raises if symmetric memory is unavailable (callers fall back to NCCL)."""
+    """Peer-visible storage of one rank: ONE torch symmetric-memory buffer with the same layout on every rank, so that
+    a peer's section is `buffer_ptrs[rank] + offset`.  ``ShardedTrainer(store=...)`` takes its buffers from it.
+    Raises if symmetric memory is unavailable."""
 
     def __init__(self, n_items, dim, world, cache_rows, device, group, stage_rows=0, sync_floats=0):
-        """``sync_floats`` > 0: also the slot / flag arrays of ``invpref_peer_allreduce`` (``ShardedTrainer.
-        enable_peer_sync``) for vectors of up to that many floats."""
+        """``stage_rows`` > 0: the sections of the push exchange -- the item shard [Iinv | Ienv], the peer-written row
+        caches and the double-buffered gradient staging of that many rows.  ``sync_floats`` > 0: the slot / flag
+        arrays of ``invpref_peer_allreduce`` (``ShardedTrainer.enable_peer_sync``) for vectors of up to that many
+        floats.  Either may be absent."""
         import torch.distributed._symmetric_memory as symm
         rows_max = (n_items + world - 1) // world
         pad = lambda n: (n + 63) // 64 * 64                      # 256-byte aligned sections
-        sizes = [("Iinv", pad(rows_max * dim)), ("Ienv", pad(rows_max * dim)),
-                 ("gcache0", pad(cache_rows * dim)), ("gcache1", pad(cache_rows * dim))]
+        sizes = []
+        self.stage_rows = int(stage_rows)
+        if self.stage_rows:
+            sizes += [("Iinv", pad(rows_max * dim)), ("Ienv", pad(rows_max * dim)),
+                      ("cache0", pad(cache_rows * dim)), ("cache1", pad(cache_rows * dim))]
+            sizes += [(f"stage{par}{t}", pad(self.stage_rows * dim)) for par in range(2) for t in range(2)]
         self.sync_floats = pad(int(sync_floats)) if sync_floats else 0
         if self.sync_floats:
             sizes += [("sync_slots", 2 * world * self.sync_floats), ("sync_flags", pad(world))]
-        if stage_rows:      # push exchange: peer-written row caches and double-buffered gradient staging
-            sizes += [("cache0", pad(cache_rows * dim)), ("cache1", pad(cache_rows * dim))]
-            sizes += [(f"stage{par}{t}", pad(stage_rows * dim)) for par in range(2) for t in range(2)]
-        self.offsets, o = {}, 0
+        self.offsets, self.sizes, o = {}, dict(sizes), 0
         for k, n in sizes:
             self.offsets[k] = o
             o += n
@@ -326,6 +318,8 @@ class SymmetricItemStorage:
         n = 1
         for d in shape:
             n *= int(d)
+        if n > self.sizes[name]:
+            raise ValueError(f"symmetric memory section {name}: {tuple(shape)} does not fit")
         o = self.offsets[name]
         return self.buf[o:o + n].view(tuple(shape))
 
@@ -349,10 +343,12 @@ class ShardedTrainer:
     """User and item tables mod-sharded by row over `world` ranks (row r of rank g holds id r*world + g)."""
 
     def __init__(self, n_users, n_items, n_envs, dim, implicit, reg_only_embed, reg_env_embed, lr, rank, world,
-                 device, cache_rows, init=None, seed=17373331, lazy=True, alloc=None, stage_rows=0):
-        """``alloc(name, shape) -> fp32 tensor``: storage for the buffers other ranks read in peer-memory mode
-        (``Iinv``, ``Ienv``, ``gcache0``, ``gcache1``), e.g. views of a torch symmetric-memory buffer; default:
-        ordinary device tensors (NCCL exchange, or simulated ranks in one process)."""
+                 device, cache_rows, init=None, seed=17373331, lazy=True, store=None, stage_rows=0):
+        """``store``: a ``SymmetricItemStorage``.  With its push sections, the item shard, the row caches and the
+        gradient staging live there (``stage_rows`` is then the store's) and the push exchange is wired
+        (``enable_push``); with its sync arrays, ``enable_peer_sync`` is wired too.  Without a store every buffer is
+        an ordinary device tensor: the NCCL exchange, or simulated ranks in one process, whose caller may wire
+        ``enable_push`` to the other ranks' tensors (``stage_rows`` > 0)."""
         self.rank, self.world, self.dev = rank, world, device
         self.U, self.I, self.K, self.D = n_users, n_items, n_envs, dim
         self.U_loc = (n_users - rank + world - 1) // world
@@ -364,21 +360,19 @@ class ShardedTrainer:
             uinv, uenv = init["Uinv"][rank::world].clone(), init["Uenv"][rank::world].clone()
             self.Iinv, self.Ienv = init["Iinv"][rank::world].clone(), init["Ienv"][rank::world].clone()
             small = [init[k].reshape(-1).clone() for k in SMALL]
-            if alloc is not None:
-                self.Iinv = alloc("Iinv", self.Iinv.shape).copy_(self.Iinv)
-                self.Ienv = alloc("Ienv", self.Ienv.shape).copy_(self.Ienv)
         else:
             g = torch.Generator(device=device).manual_seed(seed + rank)
             uinv = torch.randn((self.U_loc, dim), generator=g, **f32) * 0.01
             uenv = torch.randn((self.U_loc, dim), generator=g, **f32) * 0.01
             self.Iinv = torch.randn((self.I_loc, dim), generator=g, **f32) * 0.01
             self.Ienv = torch.randn((self.I_loc, dim), generator=g, **f32) * 0.01
-            if alloc is not None:
-                self.Iinv = alloc("Iinv", self.Iinv.shape).copy_(self.Iinv)
-                self.Ienv = alloc("Ienv", self.Ienv.shape).copy_(self.Ienv)
             g0 = torch.Generator(device=device).manual_seed(seed)          # replicated tensors: same on all ranks
             small = [torch.randn(n, generator=g0, **f32) * s for n, s in
                      ((n_envs * dim, 0.01), (n_envs * dim, 0.1), (n_envs, 0.1))]
+        peer = store is not None and store.stage_rows > 0       # the push exchange's buffers live in the store
+        if peer:
+            self.Iinv = store.alloc("Iinv", self.Iinv.shape).copy_(self.Iinv)
+            self.Ienv = store.alloc("Ienv", self.Ienv.shape).copy_(self.Ienv)
         self.mI = [torch.zeros_like(self.Iinv), torch.zeros_like(self.Ienv)]
         self.vI = [torch.zeros_like(self.Iinv), torch.zeros_like(self.Ienv)]
         self.gI = [torch.zeros_like(self.Iinv), torch.zeros_like(self.Ienv)]
@@ -390,22 +384,17 @@ class ShardedTrainer:
         views = lambda t: {"E": t[:KD].view(n_envs, dim), "W": t[KD:2 * KD].view(n_envs, dim),
                            "b": t[2 * KD:2 * KD + n_envs]}
         self.loss = self.gsmall[2 * KD + n_envs:]
-        # per-batch item cache (what the local kernels see as "the item tables") and its gradient
-        self.stage_rows = int(stage_rows)
-        if alloc is not None and self.stage_rows:
-            self.cache = [alloc(f"cache{t}", (self.cache_rows, dim)).zero_() for t in range(2)]
-        else:
-            self.cache = [torch.zeros((self.cache_rows, dim), **f32) for _ in range(2)]
-        if alloc is not None:
-            self.gcache = [alloc(f"gcache{t}", (self.cache_rows, dim)).zero_() for t in range(2)]
-        else:
-            self.gcache = [torch.zeros((self.cache_rows, dim), **f32) for _ in range(2)]
+        mk = (lambda name, shape: store.alloc(name, shape).zero_()) if peer else \
+            (lambda name, shape: torch.zeros(shape, **f32))
+        # per-batch item cache (what the local kernels see as "the item tables") and its gradient (read by the
+        # collective path only: with the push exchange the item pass stores its partials into the owners' staging)
+        self.cache = [mk(f"cache{t}", (self.cache_rows, dim)) for t in range(2)]
+        self.gcache = [torch.zeros((self.cache_rows, dim), **f32) for _ in range(2)]
         # push exchange: double-buffered staging of the ranks' partial item gradients, [parity][table]
+        self.stage_rows = store.stage_rows if store is not None else int(stage_rows)
         self.stage = None
         if self.stage_rows:
-            mk = (lambda n: alloc(n, (self.stage_rows, dim)).zero_()) if alloc is not None else \
-                (lambda n: torch.zeros((self.stage_rows, dim), **f32))
-            self.stage = [[mk(f"stage{par}{t}") for t in range(2)] for par in range(2)]
+            self.stage = [[mk(f"stage{par}{t}", (self.stage_rows, dim)) for t in range(2)] for par in range(2)]
         params = {"Uinv": uinv, "Uenv": uenv, "Iinv": self.cache[0], "Ienv": self.cache[1]}
         params.update(views(self.small))
         # lazy: the local user shard uses lazy dense Adam (bit-identical, see HotPath), so there is no dense
@@ -426,36 +415,32 @@ class ShardedTrainer:
         self._fetched = None                      # batch whose item rows are currently in the cache
         self.side = torch.cuda.Stream(device=device)
         self.phase_events = None                  # set to [] to record (name, event) marks per step (bench)
-        self.p2p = None                           # (tables ptr array, grads ptr array) once enable_p2p() ran
         self.push = None                          # push exchange state once enable_push() ran
         self.bar = torch.zeros(1, **f32)          # payload of the barrier all-reduce (peer-memory mode)
         self.sync = None                          # peer-memory all-reduce / barrier state once enable_peer_sync() ran
+        self.store = store                        # the mapped buffer outlives every pointer into it
+        if peer:
+            self.enable_push([store.ptrs("Iinv"), store.ptrs("Ienv")],
+                             [[store.ptrs(f"stage{par}{t}") for t in range(2)] for par in range(2)],
+                             [store.ptrs(f"cache{t}") for t in range(2)])
+        if store is not None and store.sync_floats:
+            self.enable_peer_sync(store.ptrs("sync_slots"), store.ptrs("sync_flags"), store.sync_floats)
 
-    def enable_p2p(self, item_inv_ptrs, item_env_ptrs, gcache0_ptrs, gcache1_ptrs):
-        """Peer-memory item exchange (NVLink loads instead of NCCL all-to-alls): the arguments are, per rank
-        0..world-1, the device address IN THIS PROCESS of that rank's Iinv / Ienv shard and of its two
-        partial-gradient caches (own rank included)."""
-        G = self.world
-        assert len(item_inv_ptrs) == len(item_env_ptrs) == len(gcache0_ptrs) == len(gcache1_ptrs) == G
-        tables = (C.c_void_p * (2 * G))(*([int(x) for x in item_inv_ptrs] + [int(x) for x in item_env_ptrs]))
-        grads = (C.c_void_p * (2 * G))(*([int(x) for x in gcache0_ptrs] + [int(x) for x in gcache1_ptrs]))
-        self.p2p = (tables, grads)
-
-    def enable_push(self, stage_ptrs, cache_ptrs):
-        """Push exchange on top of enable_p2p (which stays in use for the first fetch and for cluster_gen):
+    def enable_push(self, table_ptrs, stage_ptrs, cache_ptrs):
+        """Push exchange over peer memory (NVLink stores instead of NCCL all-to-alls): ``table_ptrs[t][rank]`` /
         ``stage_ptrs[parity][t][rank]`` / ``cache_ptrs[t][rank]`` = device address IN THIS PROCESS of rank `rank`'s
-        staging buffer / row cache of item table t (own rank included).  The item pass then stores its partial
-        gradients straight into the owners' staging buffers and the owners, after Adam, store the updated rows
-        into the requesters' caches for the next batch: no pull kernel is left on the critical path."""
+        shard / staging buffer / row cache of item table t (own rank included).  The item pass stores its partial
+        gradients straight into the owners' staging buffers and the owners, after Adam, store the updated rows into
+        the requesters' caches for the next batch.  The shards are read only where no owner has pushed the rows: the
+        first fetch of a loop or epoch and cluster_gen."""
         G = self.world
-        assert self.stage is not None and self.p2p is not None
-        base = []
-        for par in range(2):
-            flat = [int(x) for t in range(2) for x in stage_ptrs[par][t]]
-            assert len(flat) == 2 * G
-            base.append(torch.tensor(flat, dtype=torch.int64, device=self.dev))
-        caches = (C.c_void_p * (2 * G))(*[int(x) for t in range(2) for x in cache_ptrs[t]])
-        self.push = {"base": base, "caches": caches, "step": 0}
+        assert self.stage is not None
+        flat = lambda ptrs: [int(x) for t in range(2) for x in ptrs[t]]
+        assert all(len(flat(p)) == 2 * G for p in [table_ptrs, cache_ptrs] + list(stage_ptrs))
+        self.push = {"tables": (C.c_void_p * (2 * G))(*flat(table_ptrs)),
+                     "base": [torch.tensor(flat(stage_ptrs[par]), dtype=torch.int64, device=self.dev)
+                              for par in range(2)],
+                     "caches": (C.c_void_p * (2 * G))(*flat(cache_ptrs)), "step": 0}
 
     def enable_peer_sync(self, slot_ptrs, flag_ptrs, n_max):
         """The two rank-wide synchronisation points of a step (the all-reduce of the E / W / b gradients + loss sums,
@@ -523,13 +508,13 @@ class ShardedTrainer:
     def fetch_gen(self, sb: ShardedBatch):
         """All-to-all of item rows: owners pack the requested rows, requesters receive them as the cache."""
         r = sb.route
-        if self.p2p is not None:
+        if self.push is not None:
             # one kernel: every cache row is loaded straight from its owner's shard (the caller has made sure,
             # with a barrier, that all owners finished their last update)
             if r.n_cache:
                 _lib.check(self.hot.lib.invpref_fetch_rows_p2p(
-                    self.p2p[0], self.world, _lib.ptr(r.slot_owner, torch.int32), _lib.ptr(r.want_rows, torch.int64),
-                    r.n_cache, self.D, _lib.ptr(self.cache[0]), _lib.ptr(self.cache[1]), _lib.stream_ptr()),
+                    self.push["tables"], self.world, _lib.ptr(r.slot_owner, torch.int32),
+                    _lib.ptr(r.want_rows, torch.int64), r.n_cache, self.D, _lib.ptr(self.cache[0]), _lib.ptr(self.cache[1]), _lib.stream_ptr()),
                     "fetch_rows_p2p")
             return
         ns = int(r.send_rows.numel())
@@ -603,12 +588,14 @@ class ShardedTrainer:
                 yield ("all_reduce", self.gsmall)
             self._mark("grad_a2a")
             if r.spos is None:
-                r.spos = build_spos_table(r, self.world, self.I_loc)
+                r.spos = build_slot_table(r, self.world, self.I_loc,
+                                          [sum(r.send_splits[:p]) for p in range(self.world)])
             npos = None
             if next_sb is not None:
-                if next_sb.route.pos is None:
-                    next_sb.route.pos = build_pos_table(next_sb.route, self.world, self.I_loc)
-                npos = next_sb.route.pos
+                nr = next_sb.route
+                if nr.pos is None:
+                    nr.pos = build_slot_table(nr, self.world, self.I_loc, nr.peer_first)
+                npos = nr.pos
             hyper = _lib.Hyper(0, 0, 0, 0, 0, 0, self.hot.lr, self.hot.betas[0], self.hot.betas[1], self.hot.eps,
                                int(self.hot.step), 0, 0, 0, 0, 0, dyn)
             _lib.check(self.hot.lib.invpref_owner_adam_push(
@@ -636,40 +623,6 @@ class ShardedTrainer:
                 main.wait_stream(self.side)
             self._mark("sweep_wait")
             self.push["step"] += 1
-            return self.loss
-        if self.p2p is not None:
-            # Peer-memory exchange.  Barrier 1 = the all-reduce of the replicated tensors' gradients: when it
-            # returns, every rank's item pass has written its partial-gradient cache.  Then ONE kernel per rank
-            # pulls the partials of its own rows over NVLink, sums them in rank order and applies Adam.
-            if self.sync is not None:
-                self._peer_allreduce(self.gsmall)
-            else:
-                yield ("all_reduce", self.gsmall)
-            self._mark("grad_a2a")
-            if r.pos is None:
-                r.pos = build_pos_table(r, self.world, self.I_loc)
-            hyper = _lib.Hyper(0, 0, 0, 0, 0, 0, self.hot.lr, self.hot.betas[0], self.hot.betas[1], self.hot.eps,
-                               int(self.hot.step), 0, 0, 0, 0, 0)
-            _lib.check(self.hot.lib.invpref_owner_adam_p2p(
-                _lib.ptr(self.Iinv), _lib.ptr(self.Ienv), _lib.ptr(self.mI[0]), _lib.ptr(self.mI[1]),
-                _lib.ptr(self.vI[0]), _lib.ptr(self.vI[1]), self.I_loc, self.D, self.world, self.p2p[1],
-                _lib.ptr(r.pos, torch.int32), C.byref(hyper), _lib.stream_ptr()), "owner_adam_p2p")
-            self._mark("item_adam")
-            n_small = self.small.numel()
-            self.hot.adam_dense(self.small, self.msmall, self.vsmall, self.gsmall[:n_small])
-            # Barrier 2: every owner has updated its rows (and finished reading the gradient caches) before
-            # anyone fetches rows for the next batch or overwrites its cache in the next step.
-            if self.sync is not None:
-                self._peer_allreduce(None)
-            else:
-                yield ("all_reduce", self.bar)
-            self._mark("small")
-            if next_sb is not None:
-                yield from self.fetch_gen(next_sb)
-                self._fetched = next_sb
-            self._mark("prefetch_next")
-            main.wait_stream(self.side)
-            self._mark("sweep_wait")
             return self.loss
         # partial item gradients back to the owners (reverse routing)
         ns = int(r.send_rows.numel())

@@ -9,8 +9,7 @@ import torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
-from invpref_kdd_2022_b200.parallel import (DistDriver, ItemRoute, build_pos_table, build_route_gen,  # noqa: E402
-                                            build_spos_table)
+from invpref_kdd_2022_b200.parallel import DistDriver, ItemRoute, build_route_gen, build_slot_table  # noqa: E402
 
 
 def main():
@@ -67,29 +66,6 @@ def main():
     cache2 = torch.stack([shards[int(o)][int(r)] for o, r in zip(route.slot_owner.tolist(), route.want_rows.tolist())]) \
         if route.n_cache else torch.zeros((0, dim))
     ok_fetch_p2p = bool(torch.equal(cache2, cache))
-    # every rank's partial-gradient cache holds (rank + 1) in each cached row; the owner pulls through pos[p, j]
-    gcaches = gather_padded(torch.full((route.n_cache, dim), float(rank + 1)), n_items)
-    pos = build_pos_table(route, world, shard.shape[0])
-    pulled = torch.zeros_like(shard)
-    for p in range(world):
-        sl = pos[p].long()
-        has = sl >= 0
-        pulled[has] += gcaches[p][sl[has]]
-    # the same through the collective path: requesters send (rank + 1) for each cached row
-    recv2 = torch.zeros((int(route.send_rows.numel()), dim))
-
-    def back2():
-        yield ("all_to_all", recv2, torch.full((route.n_cache, dim), float(rank + 1)), route.send_splits,
-               route.recv_splits)
-
-    drv.run(back2())
-    want = torch.zeros_like(shard)
-    o = 0
-    for p in range(world):
-        n = route.send_splits[p]
-        want[route.send_rows[o:o + n]] += recv2[o:o + n]
-        o += n
-    ok_pull_p2p = bool(torch.equal(pulled, want))
 
     # ---- the PUSH exchange's tables.  Every requester "stores" (rank + 1) * 1000 + slot for cache slot c into owner
     # slot_owner[c]'s staging row push_index[c] (emulated: gather every rank's (owner, index, value) triples); the
@@ -110,7 +86,8 @@ def main():
         staging[idx] = mine[:, 2]
         writes += int(idx.numel())
     ok_push = writes == route.n_stage and not bool(torch.isnan(staging[:route.n_stage]).any())
-    spos = build_spos_table(route, world, shard.shape[0])
+    pos = build_slot_table(route, world, shard.shape[0], route.peer_first)
+    spos = build_slot_table(route, world, shard.shape[0], [sum(route.send_splits[:p]) for p in range(world)])
     # requester p's slot of my row j = pos[p, j]  =>  the staged value must be (p + 1) * 1000 + pos[p, j]
     for p in range(world):
         has = spos[p] >= 0
@@ -118,7 +95,7 @@ def main():
         got = staging[spos[p][has].long()]
         ok_push = ok_push and bool(torch.equal(got, (p + 1) * 1000.0 + pos[p][has].float()))
     print(json.dumps({"rank": rank, "fetch": ok_fetch, "back": ok_back, "fetch_p2p": ok_fetch_p2p,
-                      "pull_p2p": ok_pull_p2p, "push": ok_push, "n_cache": route.n_cache,
+                      "push": ok_push, "n_cache": route.n_cache,
                       "recv": route.recv_splits, "send": route.send_splits}), flush=True)
     dist.destroy_process_group()
 

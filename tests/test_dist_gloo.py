@@ -1,8 +1,8 @@
 """CPU, world_size 2 and 3 over gloo: the collective driver (DistDriver) and the static item routing of the
 row-sharded path (parallel.build_route_gen): every rank fetches exactly the rows its interactions need from
 their owners, and partial gradients return to the owning rank -- through the all-to-all path and through the
-tables of the peer-memory path (slot_owner / want_rows for the fetch, pos[rank][row] for the owner's pull), with the
-peers' memory emulated by all_gather."""
+tables of the push exchange (slot_owner / want_rows for the fetch, push_index / spos for the partial gradients
+staged at the owner, pos[rank][row] for the owner's row push), with the peers' memory emulated by all_gather."""
 import json
 import os
 import socket
@@ -21,7 +21,7 @@ def free_port():
 
 
 @pytest.mark.parametrize("world", [2, 3])
-def test_routing_over_gloo(world):
+def test_item_routing_over_gloo(world):
     port = free_port()
     procs = []
     for r in range(world):
@@ -37,8 +37,8 @@ def test_routing_over_gloo(world):
     assert sorted(o["rank"] for o in outs) == list(range(world))
     for o in outs:
         assert o["fetch"] and o["back"], o
-        assert o["fetch_p2p"] and o["pull_p2p"], o      # routing tables of the peer-memory exchange
-        assert o["push"], o                             # ... and of its push variant (staging rows, spos)
+        assert o["fetch_p2p"], o                        # routing tables of the peer-memory fetch
+        assert o["push"], o                             # ... and of the push exchange (staging rows, spos, pos)
         assert sum(o["recv"]) == o["n_cache"]
     # what rank a receives from b is what b sends to a
     by = {o["rank"]: o for o in outs}

@@ -22,7 +22,7 @@ def _free_port():
         return s.getsockname()[1]
 
 
-@pytest.mark.parametrize("exchange", ["push", "pull", "nccl"])
+@pytest.mark.parametrize("exchange", ["push", "nccl"])
 @pytest.mark.parametrize("case", ["explicit", "implicit"])
 def test_distributed_trainer_matches_single_gpu_on_real_ranks(case, exchange):
     n = torch.cuda.device_count()

@@ -44,11 +44,11 @@ def single_gpu(p, batches, implicit, roe, ree, lr):
     return hp, np.asarray(losses)
 
 
-@pytest.mark.parametrize("p2p", [False, True])
+@pytest.mark.parametrize("exchange", ["collective", "push"])
 @pytest.mark.parametrize("lazy", [True, False])
 @pytest.mark.parametrize("world", [2, 3])
 @pytest.mark.parametrize("implicit,roe,ree", [(False, True, False), (True, False, True)])
-def test_sharded_matches_single_gpu(world, implicit, roe, ree, lazy, p2p):
+def test_sharded_matches_single_gpu(world, implicit, roe, ree, lazy, exchange):
     from invpref_kdd_2022_b200.parallel import ShardedTrainer, SimDriver
     dev = torch.device("cuda:0")
     U, I, K, D, B = 1000, 203, 4, 64, 20000
@@ -57,12 +57,10 @@ def test_sharded_matches_single_gpu(world, implicit, roe, ree, lazy, p2p):
     batches = [(u[a:b], i[a:b], y[a:b], e[a:b], w[a:b]) for a, b in bounds]
     ref, ref_losses = single_gpu(p, batches, implicit, roe, ree, 1e-2)
     init = {k: torch.tensor(v, device=dev) for k, v in p.items()}
-    ranks = [ShardedTrainer(U, I, K, D, implicit, roe, ree, 1e-2, r, world, dev, cache_rows=I, init=init, lazy=lazy)
-             for r in range(world)]
-    if p2p:   # peer-memory exchange: the simulated ranks' buffers are plain tensors on the same device
-        for rk in ranks:
-            rk.enable_p2p([x.Iinv.data_ptr() for x in ranks], [x.Ienv.data_ptr() for x in ranks],
-                          [x.gcache[0].data_ptr() for x in ranks], [x.gcache[1].data_ptr() for x in ranks])
+    ranks = [ShardedTrainer(U, I, K, D, implicit, roe, ree, 1e-2, r, world, dev, cache_rows=I, init=init, lazy=lazy,
+                            stage_rows=2 * I if exchange == "push" else 0) for r in range(world)]
+    if exchange == "push":
+        _wire_push(ranks)
     sim = SimDriver(world)
     t = lambda a: torch.tensor(a, device=dev)
     losses = []
@@ -128,26 +126,21 @@ def test_replicated_matches_single_gpu(world):
             assert nerr(rk.params[k].cpu().numpy(), ref.params[k].cpu().numpy()) <= 2e-4, k
 
 
-def _wire(ranks, mode):
-    """Peer pointers of simulated ranks = the other ranks' tensors on the same device."""
-    if mode in ("p2p", "push"):
-        for rk in ranks:
-            rk.enable_p2p([x.Iinv.data_ptr() for x in ranks], [x.Ienv.data_ptr() for x in ranks],
-                          [x.gcache[0].data_ptr() for x in ranks], [x.gcache[1].data_ptr() for x in ranks])
-    if mode == "push":
-        for rk in ranks:
-            rk.enable_push([[[x.stage[par][t].data_ptr() for x in ranks] for t in range(2)] for par in range(2)],
-                           [[x.cache[t].data_ptr() for x in ranks] for t in range(2)])
+def _wire_push(ranks):
+    """Push exchange between simulated ranks: peer pointers = the other ranks' tensors on the same device."""
+    for rk in ranks:
+        rk.enable_push([[x.Iinv.data_ptr() for x in ranks], [x.Ienv.data_ptr() for x in ranks]],
+                       [[[x.stage[par][t].data_ptr() for x in ranks] for t in range(2)] for par in range(2)],
+                       [[x.cache[t].data_ptr() for x in ranks] for t in range(2)])
 
 
 @pytest.mark.parametrize("lazy", [True, False])
-def test_sharded_peer_memory_paths_are_bitwise_the_collective_path(lazy):
-    """Three exchanges of the item rows / partial item gradients, same arithmetic in the same (rank) order:
+def test_sharded_push_exchange_is_bitwise_the_collective_path(lazy):
+    """Two exchanges of the item rows / partial item gradients, same arithmetic in the same (rank) order:
       collective  gather_rows -> all-to-all -> cache; gradients all-to-all back -> scatter_add per rank -> adam_dense
-      p2p         invpref_fetch_rows_p2p + invpref_owner_adam_p2p (NVLink pulls)
       push        the item pass stores its partials into the owners' staging buffers (invpref_push), the owner
                   reduces from local memory and stores the updated rows into the requesters' next-batch caches
-                  (invpref_owner_adam_push): no pull kernel at all
+                  (invpref_owner_adam_push)
     must give bit-identical losses, tables and moments over several steps (double-buffered staging: 5 steps)."""
     from invpref_kdd_2022_b200.parallel import ShardedTrainer, SimDriver
     dev = torch.device("cuda:0")
@@ -156,10 +149,11 @@ def test_sharded_peer_memory_paths_are_bitwise_the_collective_path(lazy):
     init = {k: torch.tensor(v, device=dev) for k, v in p.items()}
     t = lambda a: torch.tensor(a, device=dev)
     out = []
-    for mode in ("collective", "p2p", "push"):
+    for mode in ("collective", "push"):
         ranks = [ShardedTrainer(U, I, K, D, False, True, False, 1e-2, r, world, dev, cache_rows=I, init=init,
                                 lazy=lazy, stage_rows=(2 * I if mode == "push" else 0)) for r in range(world)]
-        _wire(ranks, mode)
+        if mode == "push":
+            _wire_push(ranks)
         sim = SimDriver(world)
         losses = []
         sbs_all = []
@@ -173,7 +167,7 @@ def test_sharded_peer_memory_paths_are_bitwise_the_collective_path(lazy):
             res = sim.run_all([rk.step_gen(sb, t(e[sl])[sb.sel].contiguous(), t(w[sl])[sb.sel].contiguous(),
                                            next_sb=nx, **KW) for rk, sb, nx in zip(ranks, sbs, nxt)])
             losses.append(res[0].clone())
-        # a re-assignment after training reads the item rows through a fresh (pull) fetch
+        # a re-assignment after training reads the item rows through a fresh fetch (peer-memory loads under push)
         eps = torch.tensor(on.init_eps(K), device=dev)
         sl = slice(0, B)
         cl = sim.run_all([rk.cluster_gen(sb, None, None, t(e[sl])[sb.sel].contiguous())
