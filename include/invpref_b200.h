@@ -325,7 +325,8 @@ int invpref_hits_from_csr(const int64_t* top, int64_t b, int32_t k, const int64_
  *   rating[r, i] = predict(users[r])[i]   (models.py:393-407: sigmoid(<Uinv[u], Iinv[i]>); explicit model: no sigmoid)
  *   rating[r, mask items of users[r]] = -1024 (evaluate.py:98);  rating[r, pool items] += 1024 (evaluate.py:110)
  *   top_items[r, :] = the k items of largest rating, descending (torch.topk, evaluate.py:113; ties, which torch
- *   leaves unspecified, go to the lower item id);  hits[r, j] = top_items[r, j] in ground truth (evaluate.py:11-19);
+ *   leaves unspecified, go to the lower item id; a NaN rating, whatever its bits, ranks above +inf and ties with
+ *   every other NaN);  hits[r, j] = top_items[r, j] in ground truth (evaluate.py:11-19);
  *   n_gt[r] = size of the user's ground-truth list.
  * Lists are CSR over user ids as for invpref_mask_scores (ascending unique items per user); mask / pool / gt may be
  * NULL (no masking / no pool / no hit look-up: hits and n_gt must then be NULL).  1 <= k <= 256, k <= n_items.

@@ -66,8 +66,14 @@ __global__ void __launch_bounds__(256) hits_from_csr_kernel(const int64_t* __res
 constexpr int EV_THREADS = 256;
 constexpr int EV_MAXK = 256;
 
+// Every NaN maps to the largest key, so that NaN scores rank above +inf as in torch.topk and tie with each other
+// (lowest item id first) whatever their sign and payload; by its bits alone a NaN with the sign bit set would sort
+// below -inf.  The explicit test is also what keeps a computed NaN on top at all: nvcc folds `b | 0x80000000u` of
+// a float computed in this kernel into a negated absolute value, `FADD R, -|s|, -RZ` in the SASS, and that add
+// turns a NaN into the canonical NaN 0x7fffffff -- the key of -0.0, just below +0 (exact for every other float).
 __device__ __forceinline__ uint32_t order_key(float s) {      // ascending integer order == ascending float order
     const uint32_t b = __float_as_uint(s);
+    if (s != s) return 0xffffffffu;
     return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
 
