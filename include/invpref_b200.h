@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define INVPREF_ABI_VERSION 3
+#define INVPREF_ABI_VERSION 4
 #define INVPREF_MAX_ENVS 8      /* drivers use K = 2, 4, 5, 6 */
 #define INVPREF_MAX_DIM 256     /* drivers use D = 30, 40; synthetic config D = 64 */
 #define INVPREF_NUM_LOSSES 6    /* train.py:836-843: invariant, env_aware, envs, L2, L1, loss */
@@ -330,11 +330,26 @@ int invpref_hits_from_csr(const int64_t* top, int64_t b, int32_t k, const int64_
  *   n_gt[r] = size of the user's ground-truth list.
  * Lists are CSR over user ids as for invpref_mask_scores (ascending unique items per user); mask / pool / gt may be
  * NULL (no masking / no pool / no hit look-up: hits and n_gt must then be NULL).  1 <= k <= 256, k <= n_items.
- * top_scores (nullable): the adjusted ratings of the selected items. */
+ * top_scores (nullable): the adjusted ratings of the selected items.  From 2048 items on, the streaming top-k kernel
+ * of invpref_recommend serves this call; below, one CTA per user (same results). */
 int invpref_eval_topk(const invpref_desc* desc, const invpref_params* params, const int64_t* users, int64_t b,
                       const int64_t* mask_off, const int64_t* mask_items, const int64_t* pool_off,
                       const int64_t* pool_items, const int64_t* gt_off, const int64_t* gt_items, int32_t k,
                       int64_t* top_items, float* top_scores, uint8_t* hits, int64_t* n_gt, void* stream);
+
+/* invpref_recommend: the k best items of each of b users over the whole item table, in one kernel, without a
+ * [b, n_items] matrix: top_items[r, :] = the k items of largest score(users[r], i) = <Uinv[u], Iinv[i]> (implicit
+ * model: sigmoid of it), descending, ties to the lower item id, a NaN score above +inf; top_scores[r, :] = their
+ * scores.  excl_off / excl_items (nullable): CSR over user ids in the format of invpref_eval_topk's lists
+ * (ascending unique items per user; entries outside [0, n_items) are ignored); a user's listed items are never
+ * returned.  A user with fewer than k eligible items gets item -1 and score -inf in the trailing slots.
+ * 1 <= k <= 256, k <= n_items; b == 0 writes nothing.
+ * These are the evaluator's scores (a sum over d in ascending order, one fmaf per d, from +0), not predict()'s:
+ * they can differ from invpref_predict and InvPrefImplicit.predict in the last bits, because predict_kernel sums
+ * over a 16-lane tree and the implicit predict() is a GEMM. */
+int invpref_recommend(const invpref_desc* desc, const invpref_params* params, const int64_t* users, int64_t b,
+                      const int64_t* excl_off, const int64_t* excl_items, int32_t k, int64_t* top_items,
+                      float* top_scores, void* stream);
 
 /* ---- the same exchange over peer memory (no collective on the data path) ------------------------------------
  * Pointer arrays are HOST arrays of device pointers into the ranks' buffers, the caller's own rank included; the

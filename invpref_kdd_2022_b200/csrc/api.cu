@@ -544,6 +544,22 @@ int invpref_eval_topk(const invpref_desc* desc, const invpref_params* params, co
                             (cudaStream_t)stream);
 }
 
+int invpref_recommend(const invpref_desc* desc, const invpref_params* params, const int64_t* users, int64_t b,
+                      const int64_t* excl_off, const int64_t* excl_items, int32_t k, int64_t* top_items,
+                      float* top_scores, void* stream) {
+    Geometry g;
+    int rc = make_geometry(desc, &g);
+    if (rc != INVPREF_OK) return rc;
+    if (!params || !params->Uinv || !params->Iinv) return INVPREF_ERR_BAD_ARG;
+    if (b < 0 || k < 1 || k > 256 || k > desc->n_items || (b > 0 && (!users || !top_items || !top_scores)))
+        return INVPREF_ERR_BAD_ARG;
+    if (excl_off && !excl_items) return INVPREF_ERR_BAD_ARG;
+    if (b == 0) return INVPREF_OK;
+    return launch_topk_stream(params->Uinv, params->Iinv, desc->n_items, g.D, desc->implicit, users, b, excl_off,
+                              excl_items, nullptr, nullptr, 1, nullptr, nullptr, k, top_items, top_scores, nullptr,
+                              nullptr, (cudaStream_t)stream);
+}
+
 int invpref_fetch_rows_p2p(const float* const* tables, int32_t world, const int32_t* owner, const int64_t* rows,
                            int64_t n, int32_t dim, float* out_inv, float* out_env, void* stream) {
     if (n < 0 || dim < 1 || !tables || (n > 0 && (!owner || !rows || !out_inv || !out_env))) return INVPREF_ERR_BAD_ARG;

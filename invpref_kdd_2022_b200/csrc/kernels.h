@@ -161,10 +161,18 @@ int launch_mask_scores(float* rating, int64_t b, int64_t n_items, const int64_t*
                        const int64_t* items, float value, int add, cudaStream_t stream);
 int launch_hits_from_csr(const int64_t* top, int64_t b, int k, const int64_t* users, const int64_t* off,
                          const int64_t* items, uint8_t* hits, int64_t* n_list, cudaStream_t stream);
+// the evaluator (eval.cu): one CTA per user below 2048 items, else launch_topk_stream in EVAL mode
 int launch_eval_topk(const float* Uinv, const float* Iinv, int64_t n_items, int D, int implicit, const int64_t* users,
                      int64_t b, const int64_t* mask_off, const int64_t* mask_items, const int64_t* pool_off,
                      const int64_t* pool_items, const int64_t* gt_off, const int64_t* gt_items, int k,
                      int64_t* top_items, float* top_scores, uint8_t* hits, int64_t* n_gt, cudaStream_t stream);
+// streaming top-k (eval.cu): exclude == 0 -> list 0 = mask (-1024), list 1 = pool (+1024), hits / n_gt from gt;
+// exclude == 1 -> list 0 = items that are never candidates, no list 1, trailing slots (item -1, score -inf)
+int launch_topk_stream(const float* Uinv, const float* Iinv, int64_t n_items, int D, int implicit,
+                       const int64_t* users, int64_t b, const int64_t* list0_off, const int64_t* list0_items,
+                       const int64_t* list1_off, const int64_t* list1_items, int exclude, const int64_t* gt_off,
+                       const int64_t* gt_items, int k, int64_t* top_items, float* top_scores, uint8_t* hits,
+                       int64_t* n_gt, cudaStream_t stream);
 
 // ---- plan.cu ---------------------------------------------------------------------------------
 int build_plan_side(const int64_t* ids, const int64_t* other_ids, int64_t other_rows, const int32_t* other_seg_of,

@@ -104,14 +104,18 @@ def _read_csv(path: str, cache: bool = True) -> np.ndarray:
     return data
 
 
-def _csr(rows: np.ndarray, cols: np.ndarray, n_rows: int):
-    """Per-row sorted unique column lists as (offsets [n_rows+1], cols [nnz])."""
-    key = np.unique(rows.astype(np.int64) * (int(cols.max()) + 1 if cols.size else 1) + cols)
-    width = int(cols.max()) + 1 if cols.size else 1
-    r, c = key // width, key % width
-    off = np.zeros(n_rows + 1, dtype=np.int64)
-    np.add.at(off, r + 1, 1)
-    return np.cumsum(off), c
+def user_item_csr(users: np.ndarray, items: np.ndarray, n_users: int):
+    """Per-user sorted unique item lists as (offsets [n_users+1], items [nnz]): the list format of the evaluator and
+    of ``recommend(..., exclude=...)`` (e.g. the training pairs, to leave out items a user has already seen)."""
+    users, items = np.asarray(users), np.asarray(items)
+    width = int(items.max()) + 1 if items.size else 1
+    key = np.unique(users.astype(np.int64) * width + items)
+    off = np.zeros(n_users + 1, dtype=np.int64)
+    np.add.at(off, key // width + 1, 1)
+    return np.cumsum(off), key % width
+
+
+_csr = user_item_csr        # tests/test_gpu_drivers.py imports the earlier private name
 
 
 class ExplicitDataLoader:
@@ -152,8 +156,8 @@ class YahooImplicitBCELossDataLoader:
         self._user_num = int(max(tr[:, 0].max(), te[:, 0].max())) + 1     # dataloader.py:179-180
         self._item_num = int(max(tr[:, 1].max(), te[:, 1].max())) + 1
         pos = tr[tr[:, 2] > 0]
-        self.mask_off, self.mask_items = _csr(pos[:, 0], pos[:, 1], self._user_num)
-        self.gt_off, self.gt_items = _csr(te[:, 0], te[:, 1], self._user_num)
+        self.mask_off, self.mask_items = user_item_csr(pos[:, 0], pos[:, 1], self._user_num)
+        self.gt_off, self.gt_items = user_item_csr(te[:, 0], te[:, 1], self._user_num)
         # test users ascending (utils.py:228-233 sorts the user list)
         self.test_user_list = np.unique(te[:, 0]).tolist()
         self.test_users_tensor = torch.LongTensor(self.test_user_list).to(device)
@@ -163,7 +167,7 @@ class YahooImplicitBCELossDataLoader:
     def set_item_pool(self, pool: np.ndarray):
         """pool: int [n, >=2] (user_id, item_id) rows of test_item_pool.csv (dataloader.py:168-176)."""
         self.has_item_pool = True
-        self.pool_off, self.pool_items = _csr(pool[:, 0], pool[:, 1], self._user_num)
+        self.pool_off, self.pool_items = user_item_csr(pool[:, 0], pool[:, 1], self._user_num)
 
     def _row(self, off, items, user_id):
         return set(items[off[user_id]:off[user_id + 1]].tolist())

@@ -359,6 +359,37 @@ class HotPath:
                    "predict")
         return out
 
+    def recommend(self, users, k: int, exclude=None):
+        """``invpref_recommend``: the ``k`` best items of each user of ``users`` (int64 CUDA [b]) over the whole item
+        table -> (items int64 [b, k], scores fp32 [b, k]), score descending, ties to the lower item id.  ``exclude``:
+        ``(off, items)`` int64 CUDA tensors, CSR over user ids of items never returned; a user with fewer than ``k``
+        eligible items gets item -1 / score -inf in the trailing slots.  The scores are the evaluator's (see the
+        header): they can differ from ``predict`` in the last bits."""
+        users = users.contiguous()
+        if not users.is_cuda:
+            raise RuntimeError("recommend takes CUDA tensors only (no CPU fallback)")
+        b = users.numel()
+        if b:
+            self.check_ids(users, None, None)
+        self.flush()
+        kk = max(int(k), 1)
+        top = torch.empty((b, kk), dtype=torch.int64, device=self.device)
+        sc = torch.empty((b, kk), dtype=torch.float32, device=self.device)
+        e_off = e_items = None
+        if exclude is not None:
+            e_off, e_items = (t.contiguous() for t in exclude)
+            if e_off.dtype != torch.int64 or e_items.dtype != torch.int64 or e_off.dim() != 1 or \
+                    e_off.numel() < self.n_users + 1:
+                raise RuntimeError(f"exclude: int64 (off [n_users + 1 = {self.n_users + 1}], items) expected, got "
+                                   f"off {e_off.dtype} {tuple(e_off.shape)}, items {e_items.dtype}")
+            if not e_items.numel():
+                e_items = torch.zeros(1, dtype=torch.int64, device=self.device)        # empty lists: a valid pointer
+        p = _lib.make_params(self.params)
+        _lib.check(self.lib.invpref_recommend(C.byref(self.desc), C.byref(p), _lib.ptr(users, torch.int64), b,
+                                              _lib.ptr(e_off, torch.int64), _lib.ptr(e_items, torch.int64), int(k),
+                                              _lib.ptr(top), _lib.ptr(sc), _lib.stream_ptr()), "recommend")
+        return top, sc
+
     def backward(self, users, items, envs, alpha, g_s_inv, g_s_env, g_logp, grads: Dict[str, torch.Tensor], plan=None):
         """Accumulates the autograd gradients of ``forward`` into ``grads`` (dense, deterministic)."""
         self.flush()

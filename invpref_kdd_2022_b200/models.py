@@ -7,6 +7,7 @@ RNG stream is consumed identically).
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 from torch import nn
 
@@ -208,6 +209,21 @@ class _InvPref(nn.Module):
 
     def get_L1_reg(self, users_id, items_id, envs_id):
         return self._reg(users_id, items_id, envs_id, 1)
+
+    def recommend(self, users_id, k: int, exclude=None):
+        """The ``k`` best items of each user over the whole catalogue -> (items int64 [b, k], scores fp32 [b, k]),
+        score descending (the implicit model's sigmoid), ties to the lower item id.  ``exclude``: ``(off, items)``
+        CSR over user ids (numpy arrays or tensors, e.g. ``dataloader.user_item_csr`` of the training pairs, or an
+        implicit loader's ``mask_off`` / ``mask_items``), uploaded per call: those items are never returned, and a
+        user with fewer than ``k`` eligible items gets item -1 / score -inf in the trailing slots.  Scores can differ
+        from ``predict`` in the last bits (a different summation order)."""
+        hp = self.hot_path()
+        dev = hp.device
+        users = torch.as_tensor(users_id, dtype=torch.int64).reshape(-1).to(dev)
+        if exclude is not None:
+            exclude = tuple(torch.as_tensor(np.ascontiguousarray(x) if isinstance(x, np.ndarray) else x).to(dev)
+                            for x in exclude)
+        return hp.recommend(users, k, exclude)
 
     def cluster_predict(self, users_id, items_id, envs_id) -> torch.Tensor:
         """models.py:541-543 / 409-411: env-aware score only (the classifier pass is skipped)."""

@@ -13,7 +13,8 @@ PICK = [
     ("fused user pass (lazy, EXACT D=64 K=4)", r"upass_rows_staged_kernelILi4ELi1ELi4ELi0ELb1ELi64E"),
     ("item pass ring rows (Adam, stash, EXACT D=64 K=4)", r"bwd_rows_ring_kernelILi4ELi1ELi0ELb1ELi4ELi64E"),
     ("EM re-assignment (EXACT D=64 K=4)", r"cluster_kernelILi4ELi1ELi4ELi64E"),
-    ("fused implicit evaluator", r"eval_topk_kernel"),
+    ("streaming top-k: evaluator and recommend", r"topk_stream_kernel"),
+    ("fused implicit evaluator below 2048 items", r"eval_topk_kernel"),
     ("radix sort: rank + scatter one 8-bit digit", r"rs_scatter_kernel"),
     ("radix sort: tile histogram", r"rs_hist_kernel"),
     ("prefix sum: per-tile scan (head flags, inclusive)", r"sc_scan_kernelILi1ELb1E"),
