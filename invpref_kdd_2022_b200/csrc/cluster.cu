@@ -136,7 +136,8 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
         }
         // K sums with one scattered reduction: lanes [k * 16/NS, (k+1) * 16/NS) end up with z2[k]; each computes
         // the distance under ITS environment, then a (distance, k) butterfly picks the first minimum
-        // (torch.argmin: ties go to the lowest k) -- same values as the serial loop of train.py:853-876.
+        // (torch.argmin: ties go to the lowest k, a NaN orders below every number so the first NaN wins) -- same
+        // values as the serial loop of train.py:853-876.
         z1 = group_sum(z1, gmask);
         constexpr int NS = (KT <= 2) ? 2 : ((KT <= 4) ? 4 : 8);
         float zs[NS];
@@ -157,6 +158,9 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
         } else {
             d = INFINITY;   // padding lanes never win (an all-inf row still resolves to the lowest k)
         }
+        // torch.argmin returns the first NaN: a distance is never -inf (a square, or a BCE that is >= 0), so a NaN
+        // becomes -inf, below every number, and NaN ties still go to the lowest k
+        if (isnan(d)) d = -INFINITY;
 #pragma unroll
         for (int o = GROUP / NS; o < GROUP; o <<= 1) {
             const float d2 = __shfl_xor_sync(gmask, d, o);
@@ -312,7 +316,8 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
         }
         // K sums with one scattered reduction: lanes [k * 16/NS, (k+1) * 16/NS) end up with z2[k]; each computes
         // the distance under ITS environment, then a (distance, k) butterfly picks the first minimum
-        // (torch.argmin: ties go to the lowest k) -- same values as the serial loop of train.py:853-876.
+        // (torch.argmin: ties go to the lowest k, a NaN orders below every number so the first NaN wins) -- same
+        // values as the serial loop of train.py:853-876.
         z1 = group_sum(z1, gmask);
         constexpr int NS = (KT <= 2) ? 2 : ((KT <= 4) ? 4 : 8);
         float zs[NS];
@@ -333,6 +338,9 @@ __global__ void __launch_bounds__(BLOCK, (VEC * NV <= 4 && KT <= 4) ? 4 : 1) clu
         } else {
             d = INFINITY;   // padding lanes never win (an all-inf row still resolves to the lowest k)
         }
+        // torch.argmin returns the first NaN: a distance is never -inf (a square, or a BCE that is >= 0), so a NaN
+        // becomes -inf, below every number, and NaN ties still go to the lowest k
+        if (isnan(d)) d = -INFINITY;
 #pragma unroll
         for (int o = GROUP / NS; o < GROUP; o <<= 1) {
             const float d2 = __shfl_xor_sync(gmask, d, o);
