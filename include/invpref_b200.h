@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define INVPREF_ABI_VERSION 4
+#define INVPREF_ABI_VERSION 5
 #define INVPREF_MAX_ENVS 8      /* drivers use K = 2, 4, 5, 6 */
 #define INVPREF_MAX_DIM 256     /* drivers use D = 30, 40; synthetic config D = 64 */
 #define INVPREF_NUM_LOSSES 6    /* train.py:836-843: invariant, env_aware, envs, L2, L1, loss */
@@ -349,6 +349,37 @@ int invpref_eval_topk(const invpref_desc* desc, const invpref_params* params, co
  * over a 16-lane tree and the implicit predict() is a GEMM. */
 int invpref_recommend(const invpref_desc* desc, const invpref_params* params, const int64_t* users, int64_t b,
                       const int64_t* excl_off, const int64_t* excl_items, int32_t k, int64_t* top_items,
+                      float* top_scores, void* stream);
+
+/* invpref_similar_items: the k items most similar to each of b query items by cosine of their invariant rows
+ * (Iinv), the query item itself never returned; descending, ties to the lower id, NaN above +inf; item -1 / score
+ * -inf where fewer than k remain (k == n_items leaves the last slot so).  Repeated query ids are allowed.
+ * inv_norm: caller scratch, fp32 [n_items], overwritten with 1 / |Iinv row| first (one kernel), then read by the
+ * streaming top-k kernel of invpref_recommend.  Only Iinv is read.  1 <= k <= 256, k <= n_items; b == 0 writes
+ * nothing.  No sigmoid, on either model.
+ * Arithmetic, fixed (results do not depend on the tiling or the launch):
+ *   n2[i] = sum over d ascending of Iinv[i, d]^2, one fmaf per d from +0;  inv_norm[i] = 1.0f / sqrtf(n2[i]) (IEEE)
+ *   z = <Iinv[q], Iinv[i]> as invpref_recommend's score (one fmaf per d, ascending d, from +0)
+ *   score = (z * inv_norm[q]) * inv_norm[i] + 0.0f, each operation rounded to nearest (no contraction); the + 0
+ *   makes a -0 product +0, so a zero cosine has one key.
+ * Edge cases:
+ *   a zero row (n2 == 0) has inverse norm 0: it scores +0 against every finite row, ties going to the lower id;
+ *   a row holding a NaN or an infinity scores NaN against every row (ranked above +inf);
+ *   a finite row whose n2 overflows fp32 (entries of magnitude about 1e19 and up) gets inverse norm 1 / inf = 0 and
+ *   scores +0 (NaN where its dot product overflows too).  This limit is documented, not handled.
+ * Accuracy: the score is within about (2D + 8) * 2^-24 of the exact cosine for rows away from the fp32 range
+ * limits; ranks closer than that are ordered by the fp32 score. */
+int invpref_similar_items(const invpref_desc* desc, const invpref_params* params, const int64_t* items, int64_t b,
+                          int32_t k, float* inv_norm, int64_t* top_items, float* top_scores, void* stream);
+
+/* invpref_top_users: the k users of largest score(u, item) -- invpref_recommend's score, bit for bit: <Uinv[u],
+ * Iinv[i]>, sigmoid of it on the implicit model -- for each of b items; descending, ties to the lower user id, NaN
+ * above +inf.  excl_off / excl_users (nullable): CSR over item ids, ascending unique users per item (the transpose
+ * of invpref_recommend's lists: dataloader.user_item_csr(items, users, n_items)), entries outside [0, n_users)
+ * ignored; listed users are never returned.  An item with fewer than k eligible users gets user -1 and score -inf in
+ * the trailing slots.  1 <= k <= 256, k <= n_users; b == 0 writes nothing. */
+int invpref_top_users(const invpref_desc* desc, const invpref_params* params, const int64_t* items, int64_t b,
+                      const int64_t* excl_off, const int64_t* excl_users, int32_t k, int64_t* top_users,
                       float* top_scores, void* stream);
 
 /* ---- the same exchange over peer memory (no collective on the data path) ------------------------------------

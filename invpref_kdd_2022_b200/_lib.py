@@ -30,7 +30,7 @@ EXPORTS = (
     "invpref_check_ids", "invpref_dyn_fill", "invpref_graph_begin", "invpref_graph_end", "invpref_graph_launch",
     "invpref_graph_destroy", "invpref_graph_launches", "invpref_owner_adam_push", "invpref_eval_topk",
     "invpref_cluster_sorted", "invpref_peer_allreduce", "invpref_mt_jump_bytes", "invpref_mt_build_jumps",
-    "invpref_mt_randint", "invpref_recommend",
+    "invpref_mt_randint", "invpref_recommend", "invpref_similar_items", "invpref_top_users",
 )
 # execution order; on the fused path "forward" is empty and chunks_users / rows_users are the fused user pass
 PHASES = ("plan", "forward", "chunks_users", "rows_users", "chunks_items", "rows_items", "sweep_items",
@@ -136,6 +136,8 @@ def load() -> C.CDLL:
     lib.invpref_eval_topk.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, vp, vp, vp, vp, vp, vp, C.c_int32,
                                       vp, vp, vp, vp, vp]
     lib.invpref_recommend.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, vp, vp, C.c_int32, vp, vp, vp]
+    lib.invpref_similar_items.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, C.c_int32, vp, vp, vp, vp]
+    lib.invpref_top_users.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, vp, vp, C.c_int32, vp, vp, vp]
     lib.invpref_mask_scores.argtypes = [vp, i64, i64, vp, vp, vp, C.c_float, C.c_int32, vp]
     lib.invpref_hits_from_csr.argtypes = [vp, i64, C.c_int32, vp, vp, vp, vp, vp, vp]
     lib.invpref_mt_jump_bytes.argtypes = [C.POINTER(sz), C.POINTER(sz)]
@@ -153,7 +155,7 @@ def load() -> C.CDLL:
     return lib
 
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 ERR_ID_RANGE = -7
 
 

@@ -555,9 +555,41 @@ int invpref_recommend(const invpref_desc* desc, const invpref_params* params, co
         return INVPREF_ERR_BAD_ARG;
     if (excl_off && !excl_items) return INVPREF_ERR_BAD_ARG;
     if (b == 0) return INVPREF_OK;
-    return launch_topk_stream(params->Uinv, params->Iinv, desc->n_items, g.D, desc->implicit, users, b, excl_off,
-                              excl_items, nullptr, nullptr, 1, nullptr, nullptr, k, top_items, top_scores, nullptr,
-                              nullptr, (cudaStream_t)stream);
+    return launch_topk_stream(params->Uinv, users, b, params->Iinv, desc->n_items, g.D, desc->implicit, nullptr,
+                              excl_off, excl_items, nullptr, nullptr, 1, nullptr, nullptr, k, top_items, top_scores,
+                              nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int invpref_similar_items(const invpref_desc* desc, const invpref_params* params, const int64_t* items, int64_t b,
+                          int32_t k, float* inv_norm, int64_t* top_items, float* top_scores, void* stream) {
+    Geometry g;
+    int rc = make_geometry(desc, &g);
+    if (rc != INVPREF_OK) return rc;
+    if (!params || !params->Iinv) return INVPREF_ERR_BAD_ARG;
+    if (b < 0 || k < 1 || k > 256 || k > desc->n_items || (b > 0 && (!items || !inv_norm || !top_items || !top_scores)))
+        return INVPREF_ERR_BAD_ARG;
+    if (b == 0) return INVPREF_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = launch_row_inv_norm(params->Iinv, desc->n_items, g.D, inv_norm, st)) != INVPREF_OK) return rc;
+    return launch_topk_stream(params->Iinv, items, b, params->Iinv, desc->n_items, g.D, 0, inv_norm, nullptr,
+                              nullptr, nullptr, nullptr, 1, nullptr, nullptr, k, top_items, top_scores, nullptr,
+                              nullptr, st);
+}
+
+int invpref_top_users(const invpref_desc* desc, const invpref_params* params, const int64_t* items, int64_t b,
+                      const int64_t* excl_off, const int64_t* excl_users, int32_t k, int64_t* top_users,
+                      float* top_scores, void* stream) {
+    Geometry g;
+    int rc = make_geometry(desc, &g);
+    if (rc != INVPREF_OK) return rc;
+    if (!params || !params->Uinv || !params->Iinv) return INVPREF_ERR_BAD_ARG;
+    if (b < 0 || k < 1 || k > 256 || k > desc->n_users || (b > 0 && (!items || !top_users || !top_scores)))
+        return INVPREF_ERR_BAD_ARG;
+    if (excl_off && !excl_users) return INVPREF_ERR_BAD_ARG;
+    if (b == 0) return INVPREF_OK;
+    return launch_topk_stream(params->Iinv, items, b, params->Uinv, desc->n_users, g.D, desc->implicit, nullptr,
+                              excl_off, excl_users, nullptr, nullptr, 1, nullptr, nullptr, k, top_users, top_scores,
+                              nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int invpref_fetch_rows_p2p(const float* const* tables, int32_t world, const int32_t* owner, const int64_t* rows,

@@ -56,13 +56,21 @@ __global__ void __launch_bounds__(256) hits_from_csr_kernel(const int64_t* __res
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Streaming top-k over the whole item table for a batch of users: the evaluator (invpref_eval_topk, EVAL mode:
-// evaluate.py:88-135 + models.py:393-407) and invpref_recommend (EXCLUDE mode) -- ONE kernel, no [b, I] matrix.
+// Streaming top-k over a whole catalogue table for a batch of query rows -- ONE kernel, no [b, n] matrix:
+//   the evaluator (invpref_eval_topk, EVAL mode: evaluate.py:88-135 + models.py:393-407): users against Iinv;
+//   invpref_recommend (EXCLUDE mode): users against Iinv;  invpref_top_users (EXCLUDE mode): items against Uinv;
+//   invpref_similar_items (EXCLUDE mode, COS): items against Iinv by cosine, the query row itself skipped.
+// Below, "users" are the query rows and "items" the catalogue rows.
 //
-// A CTA owns a tile of TK_TU users (their Uinv rows in shared memory) and streams its item range in ascending tiles
+// A CTA owns a tile of TK_TU users (their rows in shared memory) and streams its item range in ascending tiles
 // of TK_TI items.  The [TU, TI] block of dot products is a register micro-tile of 4 x 4 per thread, accumulated in
 // ascending d with explicit fmaf from +0 (eval_topk_kernel's arithmetic: bit-identical scores in any tiling).  The item
 // tile is staged with cp.async, double-buffered, in chunks of at most 32 dims (large D keeps TI and the d order).
+//
+// COS (a template parameter, so that the other modes compile exactly as without it): the query ids index the
+// catalogue table itself and inv_norm holds 1 / |row| of every catalogue row (row_inv_norm_kernel).  The score is
+// (z * inv_norm[q]) * inv_norm[i] + 0, rounded after each operation (the + 0 turns a -0 product into +0: one key
+// for a zero cosine), with no sigmoid; the catalogue row equal to the query id is never a candidate.
 //
 // Exact streaming selection per user: a candidate buffer of C composites (order_key << 32 | ~item; C = 256 or 512 >= k + TK_TI), a count and
 // a threshold T (start 0; every real score has a key >= 1).  An item is appended when key > T.  Before a tile that
@@ -97,13 +105,15 @@ __device__ __forceinline__ float key_score(uint32_t k) {
 }
 
 struct TopkArgs {
-    const float *Uinv, *Iinv;
-    const int64_t* users;
+    const float *Q, *X;               // query table, catalogue table
+    const int64_t* qids;              // [b] rows of Q
+    const float* inv_norm;            // COS: [n_rows] 1 / |X row| (Q == X)
     // EVAL: list 0 = mask (score := -1024), list 1 = pool (+= 1024).  EXCLUDE: list 0 = excluded items, no list 1.
+    // Lists are CSR over query ids.
     const int64_t* off[2];
     const int64_t* items[2];
     const int64_t *gt_off, *gt_items;
-    int64_t b, n_items, slice;        // slice: items per cluster rank
+    int64_t b, n_rows, slice;         // n_rows: catalogue rows; slice: catalogue rows per cluster rank
     int D, DUS, DC, DCS, nch, k, C, implicit, exclude, vec16;
     int64_t* top_items;
     float* top_scores;
@@ -358,6 +368,7 @@ __global__ void __launch_bounds__(EV_THREADS) eval_topk_kernel(EvalArgs a) {
     if (tid == 0 && a.n_gt != nullptr) a.n_gt[r] = a.gt_off ? a.gt_off[u + 1] - a.gt_off[u] : 0;
 }
 
+template <bool COS>
 __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) {
     extern __shared__ __align__(128) unsigned char tk_smem[];
     namespace cg = cooperative_groups;
@@ -367,13 +378,15 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
     float* sU = sRing + ring_align_up(2 * TK_TI * a.DCS);                                     // [TU][DUS]
     unsigned long long* sBuf = reinterpret_cast<unsigned long long*>(sU + ring_align_up(TK_TU * a.DUS));  // [TU][C]
     uint32_t* sBits = reinterpret_cast<uint32_t*>(sBuf + (size_t)TK_TU * a.C);              // [2][TU][TI / 32]
+    int64_t* sQid = reinterpret_cast<int64_t*>(sBits + 2 * TK_TU * (TK_TI / 32));           // COS: [TU]
+    float* sQn = reinterpret_cast<float*>(sQid + TK_TU);                                     // COS: [TU]
     __shared__ uint32_t sCnt[TK_TU], sT[TK_TU];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t row0 = (int64_t)(blockIdx.x / S) * TK_TU;
     const int rows = (int)(a.b - row0 < TK_TU ? a.b - row0 : TK_TU);
     const int D = a.D, C = a.C, k = a.k;
     const int64_t lo = (int64_t)rank * a.slice;
-    const int64_t hi = lo + a.slice < a.n_items ? lo + a.slice : a.n_items;
+    const int64_t hi = lo + a.slice < a.n_rows ? lo + a.slice : a.n_rows;
     const int64_t n_tiles = hi > lo ? (hi - lo + TK_TI - 1) / TK_TI : 0;
     const int nsteps = (int)n_tiles * a.nch;
 
@@ -384,7 +397,7 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
         const int w = D - d0 < a.DC ? D - d0 : a.DC;
         const int nr = (int)(hi - i0 < TK_TI ? hi - i0 : TK_TI);
         float* dst = sRing + (size_t)(s & 1) * TK_TI * a.DCS;
-        const float* src = a.Iinv + i0 * D + d0;
+        const float* src = a.X + i0 * D + d0;
         if (a.vec16) {
             const int q = w >> 2;
             for (int p = tid; p < nr * q; p += TK_THREADS) {
@@ -405,14 +418,19 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
     __shared__ int64_t sCur[2 * TK_TU], sEnd[2 * TK_TU];
     for (int p = tid; p < TK_TU * a.DUS; p += TK_THREADS) {
         const int r = p / a.DUS, d = p - r * a.DUS;
-        sU[p] = (r < rows && d < D) ? a.Uinv[a.users[row0 + r] * D + d] : 0.f;
+        sU[p] = (r < rows && d < D) ? a.Q[a.qids[row0 + r] * D + d] : 0.f;
     }
     if (tid < TK_TU) { sCnt[tid] = 0u; sT[tid] = 0u; }
+    if (COS && tid < TK_TU) {
+        const int64_t q = tid < rows ? a.qids[row0 + tid] : -1;
+        sQid[tid] = q;
+        sQn[tid] = q >= 0 ? a.inv_norm[q] : 0.f;
+    }
     if (tid < 2 * TK_TU) {
         const int l = tid / TK_TU, r = tid % TK_TU;
         int64_t cur = 0, end = 0;
         if (a.items[l] != nullptr && r < rows) {
-            const int64_t u = a.users[row0 + r];
+            const int64_t u = a.qids[row0 + r];
             end = a.off[l][u + 1];
             cur = lower_bound(a.items[l], a.off[l][u], end, lo);
         }
@@ -493,6 +511,11 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
                     if (lane == 0) sT[r] = T;
                 }
             __syncthreads();
+            float inv_i[4];                 // COS: 1 / |row| of this thread's four tile items
+            if (COS) {
+#pragma unroll
+                for (int y = 0; y < 4; ++y) inv_i[y] = i0 + ir + 8 * y < hi ? a.inv_norm[i0 + ir + 8 * y] : 0.f;
+            }
 #pragma unroll
             for (int x = 0; x < 4; ++x) {
                 const int r = ur + 4 * x;
@@ -504,12 +527,18 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
                     const float z = acc[x][y];
                     acc[x][y] = 0.f;
                     if (r >= rows || item >= hi) continue;
-                    const bool in0 = (sBits[r * (TK_TI / 32) + (c >> 5)] >> (c & 31)) & 1u;
-                    if (a.exclude && in0) continue;
-                    float sc = a.implicit ? sigmoidf_(z) : z;
-                    if (!a.exclude) {
-                        if (in0) sc = -1024.f;
-                        if ((sBits[(TK_TU + r) * (TK_TI / 32) + (c >> 5)] >> (c & 31)) & 1u) sc += 1024.f;
+                    float sc;
+                    if (COS) {
+                        if (item == sQid[r]) continue;
+                        sc = __fadd_rn(__fmul_rn(__fmul_rn(z, sQn[r]), inv_i[y]), 0.f);   // never contracted
+                    } else {
+                        const bool in0 = (sBits[r * (TK_TI / 32) + (c >> 5)] >> (c & 31)) & 1u;
+                        if (a.exclude && in0) continue;
+                        sc = a.implicit ? sigmoidf_(z) : z;
+                        if (!a.exclude) {
+                            if (in0) sc = -1024.f;
+                            if ((sBits[(TK_TU + r) * (TK_TI / 32) + (c >> 5)] >> (c & 31)) & 1u) sc += 1024.f;
+                        }
                     }
                     const uint32_t key = order_key(sc);
                     if (key > T) {
@@ -530,7 +559,7 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
     const int share = TK_TU / S;
     for (int r = rank * share; r < (rank + 1) * share && r < rows; ++r) {
         const int64_t row = row0 + r;
-        const int64_t u = a.users[row];
+        const int64_t u = a.qids[row];
         int total = 0;
         for (int j = 0; j < S; ++j) total += (int)*cluster.map_shared_rank(&sCnt[r], j);
         for (int e = tid; e < S * k; e += TK_THREADS) {
@@ -556,7 +585,7 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
             if (a.hits != nullptr)
                 a.hits[row * k + pos] = in_sorted(a.gt_items, a.gt_off[u], a.gt_off[u + 1], item) ? 1 : 0;
         }
-        for (int p = total + tid; p < k; p += TK_THREADS) {        // EXCLUDE: fewer than k eligible items
+        for (int p = total + tid; p < k; p += TK_THREADS) {        // EXCLUDE / COS: fewer than k eligible items
             a.top_items[row * k + p] = -1;
             a.top_scores[row * k + p] = -__int_as_float(0x7f800000);
         }
@@ -565,33 +594,32 @@ __global__ void __launch_bounds__(TK_THREADS, 2) topk_stream_kernel(TopkArgs a) 
     cluster.sync();                      // no CTA exits while a peer may still read its shared memory
 }
 
-}  // namespace
+// One thread per row: inv_norm[i] = 1 / sqrtf(n2), n2 = sum over d of x[d] * x[d] as one fmaf per d in ascending d
+// from +0 (the order of the dot products above), IEEE sqrtf and division.  n2 == 0 gives 0, +inf (a non-finite
+// entry, or a sum that overflows fp32) gives 1 / inf = 0, NaN gives NaN.
+__global__ void __launch_bounds__(256) row_inv_norm_kernel(const float* __restrict__ x, int64_t n, int D, int vec4,
+                                                           float* __restrict__ inv_norm) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const float* __restrict__ row = x + i * D;
+        float n2 = 0.f;
+        if (vec4) {
+            for (int d = 0; d < D; d += 4) {
+                const float4 v = *reinterpret_cast<const float4*>(row + d);
+                n2 = fmaf(v.x, v.x, n2); n2 = fmaf(v.y, v.y, n2); n2 = fmaf(v.z, v.z, n2); n2 = fmaf(v.w, v.w, n2);
+            }
+        } else {
+            for (int d = 0; d < D; ++d) n2 = fmaf(row[d], row[d], n2);
+        }
+        inv_norm[i] = n2 == 0.f ? 0.f : 1.f / sqrtf(n2);
+    }
+}
 
-int launch_topk_stream(const float* Uinv, const float* Iinv, int64_t n_items, int D, int implicit,
-                       const int64_t* users, int64_t b, const int64_t* list0_off, const int64_t* list0_items,
-                       const int64_t* list1_off, const int64_t* list1_items, int exclude, const int64_t* gt_off,
-                       const int64_t* gt_items, int k, int64_t* top_items, float* top_scores, uint8_t* hits,
-                       int64_t* n_gt, cudaStream_t stream) {
-    TopkArgs a;
-    a.Uinv = Uinv; a.Iinv = Iinv; a.users = users;
-    a.off[0] = list0_items ? list0_off : nullptr; a.items[0] = list0_off ? list0_items : nullptr;
-    a.off[1] = list1_items ? list1_off : nullptr; a.items[1] = list1_off ? list1_items : nullptr;
-    a.gt_off = gt_off; a.gt_items = gt_items;
-    a.b = b; a.n_items = n_items; a.D = D; a.k = k; a.implicit = implicit; a.exclude = exclude;
-    a.top_items = top_items; a.top_scores = top_scores; a.hits = hits; a.n_gt = n_gt;
-    // float4 reads need a row stride of 4 floats; a stride / 4 that is odd puts the 8 rows one LDS.128 of a warp
-    // reads on 8 different 16-byte bank groups
-    const int DP = (D + 3) & ~3;
-    auto odd4 = [](int w) { return ((w >> 2) & 1) ? w : w + 4; };
-    a.DUS = odd4(DP);
-    a.nch = (DP + TK_DC - 1) / TK_DC;
-    a.DC = ((DP + a.nch - 1) / a.nch + 3) & ~3;
-    a.DCS = odd4(a.DC);
-    a.vec16 = (D % 4 == 0 && ((uintptr_t)Iinv & 15) == 0) ? 1 : 0;
-    a.C = k + TK_TI <= 256 ? 256 : 512;                  // a power of two >= k + TI
+template <bool COS>
+int launch_topk_stream_impl(TopkArgs& a, cudaStream_t stream) {
+    const int64_t b = a.b, n_rows = a.n_rows;
     const size_t smem = (size_t)ring_align_up(2 * TK_TI * a.DCS) * 4 + (size_t)ring_align_up(TK_TU * a.DUS) * 4 +
-                        (size_t)TK_TU * a.C * 8 + 2 * TK_TU * (TK_TI / 32) * 4;
-    INVPREF_SET_SMEM_ONCE(topk_stream_kernel, smem);
+                        (size_t)TK_TU * a.C * 8 + 2 * TK_TU * (TK_TI / 32) * 4 + (COS ? TK_TU * (8 + 4) : 0);
+    INVPREF_SET_SMEM_ONCE(topk_stream_kernel<COS>, smem);
     // cluster size: the slice count (1, 2, 4, 8; every slice at least one item tile) that fills the resident CTA
     // slots best, the smaller one on a tie
     // resident CTAs per SM for each shared-memory size seen (a few: D and k decide it), queried once each; one
@@ -608,7 +636,7 @@ int launch_topk_stream(const float* Uinv, const float* Iinv, int64_t n_items, in
     for (int j = 0; j < n_occ && per_sm == 0; ++j)
         if (occ_smem[j] == smem) per_sm = occ_ctas[j];
     if (per_sm == 0) {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, topk_stream_kernel, TK_THREADS, smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, topk_stream_kernel<COS>, TK_THREADS, smem);
         per_sm = per_sm > 0 ? per_sm : 1;
         if (n_occ < 16) { occ_smem[n_occ] = smem; occ_ctas[n_occ] = per_sm; ++n_occ; }
     }
@@ -616,12 +644,12 @@ int launch_topk_stream(const float* Uinv, const float* Iinv, int64_t n_items, in
     const int64_t tiles = (b + TK_TU - 1) / TK_TU;
     int S = 1;
     double best = 0.0;
-    for (int s = 1; s <= TK_MAX_SLICES && (s == 1 || n_items >= (int64_t)s * TK_TI); s *= 2) {
+    for (int s = 1; s <= TK_MAX_SLICES && (s == 1 || n_rows >= (int64_t)s * TK_TI); s *= 2) {
         const int64_t ctas = tiles * s;
         const double fill = (double)ctas / (double)(((ctas + slots - 1) / slots) * slots);
         if (fill > best + 1e-9) { best = fill; S = s; }
     }
-    a.slice = (n_items + S - 1) / S;
+    a.slice = (n_rows + S - 1) / S;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(tiles * S));
     cfg.blockDim = dim3(TK_THREADS);
@@ -634,9 +662,45 @@ int launch_topk_stream(const float* Uinv, const float* Iinv, int64_t n_items, in
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, topk_stream_kernel, a);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, topk_stream_kernel<COS>, a);
     count_launch();
     return (e == cudaSuccess && cudaGetLastError() == cudaSuccess) ? INVPREF_OK : INVPREF_ERR_CUDA;
+}
+
+}  // namespace
+
+int launch_topk_stream(const float* Q, const int64_t* qids, int64_t b, const float* X, int64_t n_rows, int D,
+                       int implicit, const float* inv_norm, const int64_t* list0_off, const int64_t* list0_items,
+                       const int64_t* list1_off, const int64_t* list1_items, int exclude, const int64_t* gt_off,
+                       const int64_t* gt_items, int k, int64_t* top_items, float* top_scores, uint8_t* hits,
+                       int64_t* n_gt, cudaStream_t stream) {
+    TopkArgs a;
+    a.Q = Q; a.X = X; a.qids = qids; a.inv_norm = inv_norm;
+    a.off[0] = list0_items ? list0_off : nullptr; a.items[0] = list0_off ? list0_items : nullptr;
+    a.off[1] = list1_items ? list1_off : nullptr; a.items[1] = list1_off ? list1_items : nullptr;
+    a.gt_off = gt_off; a.gt_items = gt_items;
+    a.b = b; a.n_rows = n_rows; a.D = D; a.k = k; a.implicit = implicit; a.exclude = exclude;
+    a.top_items = top_items; a.top_scores = top_scores; a.hits = hits; a.n_gt = n_gt;
+    // float4 reads need a row stride of 4 floats; a stride / 4 that is odd puts the 8 rows one LDS.128 of a warp
+    // reads on 8 different 16-byte bank groups
+    const int DP = (D + 3) & ~3;
+    auto odd4 = [](int w) { return ((w >> 2) & 1) ? w : w + 4; };
+    a.DUS = odd4(DP);
+    a.nch = (DP + TK_DC - 1) / TK_DC;
+    a.DC = ((DP + a.nch - 1) / a.nch + 3) & ~3;
+    a.DCS = odd4(a.DC);
+    a.vec16 = (D % 4 == 0 && ((uintptr_t)X & 15) == 0) ? 1 : 0;
+    a.C = k + TK_TI <= 256 ? 256 : 512;                  // a power of two >= k + TI
+    return inv_norm ? launch_topk_stream_impl<true>(a, stream) : launch_topk_stream_impl<false>(a, stream);
+}
+
+int launch_row_inv_norm(const float* x, int64_t n, int D, float* inv_norm, cudaStream_t stream) {
+    const int64_t need = (n + 255) / 256;
+    const int grid = (int)(need < 1 ? 1 : (need < 148 * 16 ? need : 148 * 16));
+    const int vec4 = (D % 4 == 0 && ((uintptr_t)x & 15) == 0) ? 1 : 0;
+    row_inv_norm_kernel<<<grid, 256, 0, stream>>>(x, n, D, vec4, inv_norm);
+    count_launch();
+    return cudaGetLastError() == cudaSuccess ? INVPREF_OK : INVPREF_ERR_CUDA;
 }
 
 int launch_mask_scores(float* rating, int64_t b, int64_t n_items, const int64_t* users, const int64_t* off,
@@ -665,8 +729,9 @@ int launch_eval_topk(const float* Uinv, const float* Iinv, int64_t n_items, int 
     // kernel (Yahoo-implicit: 1 000 items, b = 1 024); from there on the user tiles' shared item reads win
     // (MovieLens: 3 706 items, MIND: 51 283; profiles/r3_topk_stream*.json).  Both give the same results.
     if (n_items >= EV_STREAM_MIN_ITEMS)
-        return launch_topk_stream(Uinv, Iinv, n_items, D, implicit, users, b, mask_off, mask_items, pool_off,
-                                  pool_items, 0, gt_off, gt_items, k, top_items, top_scores, hits, n_gt, stream);
+        return launch_topk_stream(Uinv, users, b, Iinv, n_items, D, implicit, nullptr, mask_off, mask_items,
+                                  pool_off, pool_items, 0, gt_off, gt_items, k, top_items, top_scores, hits, n_gt,
+                                  stream);
     EvalArgs a;
     a.Uinv = Uinv; a.Iinv = Iinv; a.users = users; a.mask_off = mask_off; a.mask_items = mask_items;
     a.pool_off = pool_off; a.pool_items = pool_items; a.gt_off = gt_off; a.gt_items = gt_items;

@@ -166,13 +166,19 @@ int launch_eval_topk(const float* Uinv, const float* Iinv, int64_t n_items, int 
                      int64_t b, const int64_t* mask_off, const int64_t* mask_items, const int64_t* pool_off,
                      const int64_t* pool_items, const int64_t* gt_off, const int64_t* gt_items, int k,
                      int64_t* top_items, float* top_scores, uint8_t* hits, int64_t* n_gt, cudaStream_t stream);
-// streaming top-k (eval.cu): exclude == 0 -> list 0 = mask (-1024), list 1 = pool (+1024), hits / n_gt from gt;
-// exclude == 1 -> list 0 = items that are never candidates, no list 1, trailing slots (item -1, score -inf)
-int launch_topk_stream(const float* Uinv, const float* Iinv, int64_t n_items, int D, int implicit,
-                       const int64_t* users, int64_t b, const int64_t* list0_off, const int64_t* list0_items,
+// streaming top-k (eval.cu) of the b query rows Q[qids[r]] over the n_rows rows of the catalogue table X: score =
+// <query row, catalogue row> (sigmoid of it if implicit); lists are CSR over query ids.
+// exclude == 0 -> list 0 = mask (-1024), list 1 = pool (+1024), hits / n_gt from gt;
+// exclude == 1 -> list 0 = catalogue rows that are never candidates, no list 1, trailing slots (item -1, score -inf).
+// inv_norm != NULL -> cosine (Q == X, qids index X, inv_norm [n_rows] from launch_row_inv_norm), no sigmoid, catalogue
+// row qids[r] never a candidate of query r; pass exclude == 1 and no lists.
+int launch_topk_stream(const float* Q, const int64_t* qids, int64_t b, const float* X, int64_t n_rows, int D,
+                       int implicit, const float* inv_norm, const int64_t* list0_off, const int64_t* list0_items,
                        const int64_t* list1_off, const int64_t* list1_items, int exclude, const int64_t* gt_off,
                        const int64_t* gt_items, int k, int64_t* top_items, float* top_scores, uint8_t* hits,
                        int64_t* n_gt, cudaStream_t stream);
+// inv_norm[i] = 1 / sqrtf(sum_d x[i, d]^2) for the n rows of x [n, D] (row_inv_norm_kernel: order and edge cases)
+int launch_row_inv_norm(const float* x, int64_t n, int D, float* inv_norm, cudaStream_t stream);
 
 // ---- plan.cu ---------------------------------------------------------------------------------
 int build_plan_side(const int64_t* ids, const int64_t* other_ids, int64_t other_rows, const int32_t* other_seg_of,

@@ -106,7 +106,9 @@ def _read_csv(path: str, cache: bool = True) -> np.ndarray:
 
 def user_item_csr(users: np.ndarray, items: np.ndarray, n_users: int):
     """Per-user sorted unique item lists as (offsets [n_users+1], items [nnz]): the list format of the evaluator and
-    of ``recommend(..., exclude=...)`` (e.g. the training pairs, to leave out items a user has already seen)."""
+    of ``recommend(..., exclude=...)`` (e.g. the training pairs, to leave out items a user has already seen).  With
+    the roles swapped, ``user_item_csr(items, users, n_items)`` gives the users of each item: the ``exclude`` lists
+    of ``top_users`` (users who already interacted with an item)."""
     users, items = np.asarray(users), np.asarray(items)
     width = int(items.max()) + 1 if items.size else 1
     key = np.unique(users.astype(np.int64) * width + items)

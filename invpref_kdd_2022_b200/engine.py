@@ -365,30 +365,79 @@ class HotPath:
         ``(off, items)`` int64 CUDA tensors, CSR over user ids of items never returned; a user with fewer than ``k``
         eligible items gets item -1 / score -inf in the trailing slots.  The scores are the evaluator's (see the
         header): they can differ from ``predict`` in the last bits."""
-        users = users.contiguous()
-        if not users.is_cuda:
-            raise RuntimeError("recommend takes CUDA tensors only (no CPU fallback)")
+        users = self._query_ids(users, "recommend")
         b = users.numel()
         if b:
             self.check_ids(users, None, None)
         self.flush()
-        kk = max(int(k), 1)
-        top = torch.empty((b, kk), dtype=torch.int64, device=self.device)
-        sc = torch.empty((b, kk), dtype=torch.float32, device=self.device)
-        e_off = e_items = None
-        if exclude is not None:
-            e_off, e_items = (t.contiguous() for t in exclude)
-            if e_off.dtype != torch.int64 or e_items.dtype != torch.int64 or e_off.dim() != 1 or \
-                    e_off.numel() < self.n_users + 1:
-                raise RuntimeError(f"exclude: int64 (off [n_users + 1 = {self.n_users + 1}], items) expected, got "
-                                   f"off {e_off.dtype} {tuple(e_off.shape)}, items {e_items.dtype}")
-            if not e_items.numel():
-                e_items = torch.zeros(1, dtype=torch.int64, device=self.device)        # empty lists: a valid pointer
+        top, sc = self._topk_out(b, k)
+        e_off, e_items = self._exclusion_csr(exclude, self.n_users, "n_users")
         p = _lib.make_params(self.params)
         _lib.check(self.lib.invpref_recommend(C.byref(self.desc), C.byref(p), _lib.ptr(users, torch.int64), b,
                                               _lib.ptr(e_off, torch.int64), _lib.ptr(e_items, torch.int64), int(k),
                                               _lib.ptr(top), _lib.ptr(sc), _lib.stream_ptr()), "recommend")
         return top, sc
+
+    def similar_items(self, items, k: int):
+        """``invpref_similar_items``: the ``k`` items nearest to each item of ``items`` (int64 CUDA [b]) by cosine of
+        the invariant item rows, the query item itself left out -> (items int64 [b, k], scores fp32 [b, k]), cosine
+        descending, ties to the lower item id, item -1 / score -inf where fewer than ``k`` remain.  Reads only the
+        item table, which lazy Adam never defers: no flush."""
+        items = self._query_ids(items, "similar_items")
+        b = items.numel()
+        if b:
+            self.check_ids(None, items, None)
+        top, sc = self._topk_out(b, k)
+        inv_norm = torch.empty(self.n_items, dtype=torch.float32, device=self.device)    # the table changes per call
+        p = _lib.make_params(self.params)
+        _lib.check(self.lib.invpref_similar_items(C.byref(self.desc), C.byref(p), _lib.ptr(items, torch.int64), b,
+                                                  int(k), _lib.ptr(inv_norm), _lib.ptr(top), _lib.ptr(sc),
+                                                  _lib.stream_ptr()), "similar_items")
+        return top, sc
+
+    def top_users(self, items, k: int, exclude=None):
+        """``invpref_top_users``: the ``k`` users of largest score for each item of ``items`` (int64 CUDA [b]) ->
+        (users int64 [b, k], scores fp32 [b, k]), score descending, ties to the lower user id; the scores are
+        ``recommend``'s, bit for bit.  ``exclude``: ``(off, users)`` int64 CUDA tensors, CSR over item ids of users
+        never returned (``dataloader.user_item_csr(items, users, n_items)``); an item with fewer than ``k`` eligible
+        users gets user -1 / score -inf in the trailing slots."""
+        items = self._query_ids(items, "top_users")
+        b = items.numel()
+        if b:
+            self.check_ids(None, items, None)
+        self.flush()
+        top, sc = self._topk_out(b, k)
+        e_off, e_users = self._exclusion_csr(exclude, self.n_items, "n_items")
+        p = _lib.make_params(self.params)
+        _lib.check(self.lib.invpref_top_users(C.byref(self.desc), C.byref(p), _lib.ptr(items, torch.int64), b,
+                                              _lib.ptr(e_off, torch.int64), _lib.ptr(e_users, torch.int64), int(k),
+                                              _lib.ptr(top), _lib.ptr(sc), _lib.stream_ptr()), "top_users")
+        return top, sc
+
+    @staticmethod
+    def _query_ids(ids, what):
+        ids = ids.contiguous()
+        if not ids.is_cuda:
+            raise RuntimeError(f"{what} takes CUDA tensors only (no CPU fallback)")
+        return ids
+
+    def _topk_out(self, b, k):
+        kk = max(int(k), 1)          # k outside [1, 256] is the library's BAD_ARG
+        return (torch.empty((b, kk), dtype=torch.int64, device=self.device),
+                torch.empty((b, kk), dtype=torch.float32, device=self.device))
+
+    def _exclusion_csr(self, exclude, n_query_rows, name):
+        """(off, ids) of a CSR exclusion list over ``n_query_rows`` query ids, checked; (None, None) without one."""
+        if exclude is None:
+            return None, None
+        e_off, e_ids = (t.contiguous() for t in exclude)
+        if e_off.dtype != torch.int64 or e_ids.dtype != torch.int64 or e_off.dim() != 1 or \
+                e_off.numel() < n_query_rows + 1:
+            raise RuntimeError(f"exclude: int64 (off [{name} + 1 = {n_query_rows + 1}], ids) expected, got "
+                               f"off {e_off.dtype} {tuple(e_off.shape)}, ids {e_ids.dtype}")
+        if not e_ids.numel():
+            e_ids = torch.zeros(1, dtype=torch.int64, device=self.device)        # empty lists: a valid pointer
+        return e_off, e_ids
 
     def backward(self, users, items, envs, alpha, g_s_inv, g_s_env, g_logp, grads: Dict[str, torch.Tensor], plan=None):
         """Accumulates the autograd gradients of ``forward`` into ``grads`` (dense, deterministic)."""

@@ -218,18 +218,42 @@ class _InvPref(nn.Module):
         user with fewer than ``k`` eligible items gets item -1 / score -inf in the trailing slots.  Scores can differ
         from ``predict`` in the last bits (a different summation order)."""
         hp = self.hot_path()
-        dev = hp.device
-        users = torch.as_tensor(users_id, dtype=torch.int64).reshape(-1).to(dev)
-        if exclude is not None:
-            exclude = tuple(torch.as_tensor(np.ascontiguousarray(x) if isinstance(x, np.ndarray) else x).to(dev)
-                            for x in exclude)
-        return hp.recommend(users, k, exclude)
+        return hp.recommend(_ids_on(users_id, hp.device), k, _csr_on(exclude, hp.device))
+
+    def similar_items(self, items_id, k: int):
+        """The ``k`` items nearest to each given item by cosine of the invariant item embeddings -> (items int64
+        [b, k], cosines fp32 [b, k]), descending, ties to the lower item id; an item is never its own neighbour, so
+        ``k == item_num`` ends in item -1 / score -inf.  No sigmoid on either model.  Zero rows score +0 against every
+        finite row; a row holding NaN or inf scores NaN (ranked first).  ``items_id``: numpy array or tensor."""
+        hp = self.hot_path()
+        return hp.similar_items(_ids_on(items_id, hp.device), k)
+
+    def top_users(self, items_id, k: int, exclude=None):
+        """The ``k`` users of largest score for each given item -> (users int64 [b, k], scores fp32 [b, k]), score
+        descending, ties to the lower user id; the scores are ``recommend``'s for the same (user, item), bit for bit.
+        ``exclude``: ``(off, users)`` CSR over item ids (numpy arrays or tensors), e.g. the users who already
+        interacted with each item, ``dataloader.user_item_csr(items, users, item_num)`` of the training pairs: those
+        users are never returned, and an item with fewer than ``k`` eligible users gets user -1 / score -inf in the
+        trailing slots."""
+        hp = self.hot_path()
+        return hp.top_users(_ids_on(items_id, hp.device), k, _csr_on(exclude, hp.device))
 
     def cluster_predict(self, users_id, items_id, envs_id) -> torch.Tensor:
         """models.py:541-543 / 409-411: env-aware score only (the classifier pass is skipped)."""
         hp = self.hot_path()
         _, s_env, _ = hp.forward(users_id.contiguous(), items_id.contiguous(), envs_id.contiguous(), want_logp=False)
         return s_env
+
+
+def _ids_on(ids, dev) -> torch.Tensor:
+    return torch.as_tensor(ids, dtype=torch.int64).reshape(-1).to(dev)
+
+
+def _csr_on(csr, dev):
+    """(off, ids) numpy arrays or tensors -> tensors on `dev` (uploaded per call); None stays None."""
+    if csr is None:
+        return None
+    return tuple(torch.as_tensor(np.ascontiguousarray(x) if isinstance(x, np.ndarray) else x).to(dev) for x in csr)
 
 
 class BasicRecommender(nn.Module):
