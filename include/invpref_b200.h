@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define INVPREF_ABI_VERSION 5
+#define INVPREF_ABI_VERSION 6
 #define INVPREF_MAX_ENVS 8      /* drivers use K = 2, 4, 5, 6 */
 #define INVPREF_MAX_DIM 256     /* drivers use D = 30, 40; synthetic config D = 64 */
 #define INVPREF_NUM_LOSSES 6    /* train.py:836-843: invariant, env_aware, envs, L2, L1, loss */
@@ -381,6 +381,60 @@ int invpref_similar_items(const invpref_desc* desc, const invpref_params* params
 int invpref_top_users(const invpref_desc* desc, const invpref_params* params, const int64_t* items, int64_t b,
                       const int64_t* excl_off, const int64_t* excl_users, int32_t k, int64_t* top_users,
                       float* top_scores, void* stream);
+
+/* invpref_fold_in_users: invariant user rows for b users who are not in the tables, from their histories, with the
+ * item table fixed.  Row r's history is the pairs (items[p], scores[p]) for p in [off[r], off[r + 1]) (CSR, off
+ * [b + 1]; duplicate ids count as separate observations).  With V = Iinv and z_p = <u, V[items[p]]>, rows[r, :] is
+ * the fp32 rounding of the u that minimises
+ *   explicit model:  1/2 sum_p (z_p - y_p)^2 + l2/2 |u|^2     (the invariant branch of the MSE loss, plus a ridge term)
+ *   implicit model:  sum_p [softplus(z_p) - y_p z_p] + l2/2 |u|^2   (BCE of sigmoid(z), without nn.BCELoss's clamp
+ *                    of the log at -100; labels y_p may be fractional in [0, 1])
+ * so that invpref_recommend_rows ranks the catalogue for it as invpref_recommend ranks a trained user.  l2 is a
+ * per-row ridge: the training L2 term is a per-batch mean and does not map onto it, so there is no default.
+ * Method (one CTA per row, no global workspace):
+ *   explicit: (Vh^T Vh + l2 I) u = Vh^T y, Vh the history's rows of V, by an LDL^T (square-root-free Cholesky)
+ *   factorisation and two triangular solves; iters[r] = 1.
+ *   implicit: damped Newton from u = 0.  Each step solves (H + l2 I) dl = -g, H = sum_p s_p (1 - s_p) v_p v_p^T,
+ *   g = sum_p (s_p - y_p) v_p + l2 u, s_p = sigmoid(z_p), the same way.  If max|dl| <= 2^-30 * max(1, max|u|) the full
+ *   step is taken and the row has converged (iters[r] = the number of steps, in [1, max_iter]).  Otherwise the step
+ *   length t = 1, 1/2, ..., 2^-30 is the first that satisfies Armijo, f(u + t dl) - f(u) <= 1e-4 t g^T dl (the last
+ *   one if none does), the difference summed per history entry as log1p(s_p expm1(t dz_p)) - y_p t dz_p plus the
+ *   ridge term, which keeps the decrease visible near the optimum.  A row still going after max_iter steps is
+ *   written as it stands with iters[r] = -max_iter.
+ * Arithmetic: table rows and scores are read as fp32; every product, sum, factorisation and Newton update is fp64,
+ * and the history sums run in CSR order without atomics.  Row r's result depends only on its history, l2, max_iter
+ * and V: not on b, on its position in the batch or on the launch geometry, bit for bit.
+ * Edge cases: an empty history gives the zero row and iters 0.  A NaN or infinite score or table row in a history
+ * (or an overflow while solving) makes that row NaN (iters -max_iter on the implicit model) and no other.  History
+ * ids outside [0, n_items) are skipped.  iters is nullable.
+ * Limits: 1 <= dim <= 128 (the fp64 triangle of the system lives in shared memory: 66 KB at D = 128), else
+ * INVPREF_ERR_BAD_DIM; l2 finite and > 0 (every system is then symmetric positive definite) and max_iter >= 1, else
+ * INVPREF_ERR_BAD_ARG.  b == 0 writes nothing.  No launch on an error.
+ * Accuracy: the explicit row is within 1/2 ulp (fp32) plus about (D + n) * cond * 2^-53 * max|u| of the exact solution,
+ * n the history length and cond the condition number of the system. */
+int invpref_fold_in_users(const invpref_desc* desc, const invpref_params* params, const int64_t* off,
+                          const int64_t* items, const float* scores, int64_t b, double l2, int32_t max_iter,
+                          float* rows, int32_t* iters, void* stream);
+
+/* invpref_fold_in_items: the same for items that are not in the tables, against the user table (V = Uinv, ids in
+ * [0, n_users)): invariant item rows from (user, score) histories, for invpref_top_users_rows. */
+int invpref_fold_in_items(const invpref_desc* desc, const invpref_params* params, const int64_t* off,
+                          const int64_t* users, const float* scores, int64_t b, double l2, int32_t max_iter,
+                          float* rows, int32_t* iters, void* stream);
+
+/* invpref_recommend_rows: invpref_recommend for query rows the caller supplies (e.g. folded-in users): query r is the
+ * row rows[row_ids[r], :] of a fp32 table [*, dim]; its scores against Iinv are invpref_recommend's, bit for bit
+ * (sigmoid on the implicit model), so recommend_rows(Uinv, users) == recommend(users).  excl_off / excl_items: CSR
+ * over row ids in invpref_recommend's format.  Same limits as invpref_recommend; only Iinv is read from params. */
+int invpref_recommend_rows(const invpref_desc* desc, const invpref_params* params, const float* rows,
+                           const int64_t* row_ids, int64_t b, const int64_t* excl_off, const int64_t* excl_items,
+                           int32_t k, int64_t* top_items, float* top_scores, void* stream);
+
+/* invpref_top_users_rows: invpref_top_users for caller-supplied item rows (e.g. folded-in items), against Uinv;
+ * top_users_rows(Iinv, items) == top_users(items), bit for bit.  Exclusion CSR over row ids. */
+int invpref_top_users_rows(const invpref_desc* desc, const invpref_params* params, const float* rows,
+                           const int64_t* row_ids, int64_t b, const int64_t* excl_off, const int64_t* excl_users,
+                           int32_t k, int64_t* top_users, float* top_scores, void* stream);
 
 /* ---- the same exchange over peer memory (no collective on the data path) ------------------------------------
  * Pointer arrays are HOST arrays of device pointers into the ranks' buffers, the caller's own rank included; the

@@ -31,6 +31,7 @@ EXPORTS = (
     "invpref_graph_destroy", "invpref_graph_launches", "invpref_owner_adam_push", "invpref_eval_topk",
     "invpref_cluster_sorted", "invpref_peer_allreduce", "invpref_mt_jump_bytes", "invpref_mt_build_jumps",
     "invpref_mt_randint", "invpref_recommend", "invpref_similar_items", "invpref_top_users",
+    "invpref_fold_in_users", "invpref_fold_in_items", "invpref_recommend_rows", "invpref_top_users_rows",
 )
 # execution order; on the fused path "forward" is empty and chunks_users / rows_users are the fused user pass
 PHASES = ("plan", "forward", "chunks_users", "rows_users", "chunks_items", "rows_items", "sweep_items",
@@ -138,6 +139,11 @@ def load() -> C.CDLL:
     lib.invpref_recommend.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, vp, vp, C.c_int32, vp, vp, vp]
     lib.invpref_similar_items.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, C.c_int32, vp, vp, vp, vp]
     lib.invpref_top_users.argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, i64, vp, vp, C.c_int32, vp, vp, vp]
+    for name in ("invpref_fold_in_users", "invpref_fold_in_items"):
+        getattr(lib, name).argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, vp, vp, i64, C.c_double, C.c_int32, vp,
+                                       vp, vp]
+    for name in ("invpref_recommend_rows", "invpref_top_users_rows"):
+        getattr(lib, name).argtypes = [C.POINTER(Desc), C.POINTER(Params), vp, vp, i64, vp, vp, C.c_int32, vp, vp, vp]
     lib.invpref_mask_scores.argtypes = [vp, i64, i64, vp, vp, vp, C.c_float, C.c_int32, vp]
     lib.invpref_hits_from_csr.argtypes = [vp, i64, C.c_int32, vp, vp, vp, vp, vp, vp]
     lib.invpref_mt_jump_bytes.argtypes = [C.POINTER(sz), C.POINTER(sz)]
@@ -155,7 +161,8 @@ def load() -> C.CDLL:
     return lib
 
 
-ABI_VERSION = 5
+ABI_VERSION = 6
+FOLD_IN_MAX_DIM = 128
 ERR_ID_RANGE = -7
 
 

@@ -592,6 +592,67 @@ int invpref_top_users(const invpref_desc* desc, const invpref_params* params, co
                               nullptr, nullptr, (cudaStream_t)stream);
 }
 
+static int fold_in(const invpref_desc* desc, const float* V, int64_t n_cat, const int64_t* off, const int64_t* ids,
+                   const float* scores, int64_t b, double l2, int32_t max_iter, float* rows, int32_t* iters,
+                   void* stream) {
+    if (!desc) return INVPREF_ERR_BAD_ARG;
+    if (desc->dim < 1 || desc->dim > fold_in_max_dim()) return INVPREF_ERR_BAD_DIM;
+    if (desc->n_users < 1 || desc->n_items < 1 || !V) return INVPREF_ERR_BAD_ARG;
+    if (!(l2 > 0.0) || !isfinite(l2) || max_iter < 1 || b < 0) return INVPREF_ERR_BAD_ARG;
+    if (b > 0 && (!off || !ids || !scores || !rows)) return INVPREF_ERR_BAD_ARG;
+    if (b == 0) return INVPREF_OK;
+    return launch_fold_in(V, n_cat, desc->dim, desc->implicit, off, ids, scores, b, l2, max_iter, rows, iters,
+                          (cudaStream_t)stream);
+}
+
+int invpref_fold_in_users(const invpref_desc* desc, const invpref_params* params, const int64_t* off,
+                          const int64_t* items, const float* scores, int64_t b, double l2, int32_t max_iter,
+                          float* rows, int32_t* iters, void* stream) {
+    if (!desc || !params) return INVPREF_ERR_BAD_ARG;
+    return fold_in(desc, params->Iinv, desc->n_items, off, items, scores, b, l2, max_iter, rows, iters, stream);
+}
+
+int invpref_fold_in_items(const invpref_desc* desc, const invpref_params* params, const int64_t* off,
+                          const int64_t* users, const float* scores, int64_t b, double l2, int32_t max_iter,
+                          float* rows, int32_t* iters, void* stream) {
+    if (!desc || !params) return INVPREF_ERR_BAD_ARG;
+    return fold_in(desc, params->Uinv, desc->n_users, off, users, scores, b, l2, max_iter, rows, iters, stream);
+}
+
+int invpref_recommend_rows(const invpref_desc* desc, const invpref_params* params, const float* rows,
+                           const int64_t* row_ids, int64_t b, const int64_t* excl_off, const int64_t* excl_items,
+                           int32_t k, int64_t* top_items, float* top_scores, void* stream) {
+    Geometry g;
+    int rc = make_geometry(desc, &g);
+    if (rc != INVPREF_OK) return rc;
+    if (!params || !params->Iinv) return INVPREF_ERR_BAD_ARG;
+    if (b < 0 || k < 1 || k > 256 || k > desc->n_items ||
+        (b > 0 && (!rows || !row_ids || !top_items || !top_scores)))
+        return INVPREF_ERR_BAD_ARG;
+    if (excl_off && !excl_items) return INVPREF_ERR_BAD_ARG;
+    if (b == 0) return INVPREF_OK;
+    return launch_topk_stream(rows, row_ids, b, params->Iinv, desc->n_items, g.D, desc->implicit, nullptr, excl_off,
+                              excl_items, nullptr, nullptr, 1, nullptr, nullptr, k, top_items, top_scores, nullptr,
+                              nullptr, (cudaStream_t)stream);
+}
+
+int invpref_top_users_rows(const invpref_desc* desc, const invpref_params* params, const float* rows,
+                           const int64_t* row_ids, int64_t b, const int64_t* excl_off, const int64_t* excl_users,
+                           int32_t k, int64_t* top_users, float* top_scores, void* stream) {
+    Geometry g;
+    int rc = make_geometry(desc, &g);
+    if (rc != INVPREF_OK) return rc;
+    if (!params || !params->Uinv) return INVPREF_ERR_BAD_ARG;
+    if (b < 0 || k < 1 || k > 256 || k > desc->n_users ||
+        (b > 0 && (!rows || !row_ids || !top_users || !top_scores)))
+        return INVPREF_ERR_BAD_ARG;
+    if (excl_off && !excl_users) return INVPREF_ERR_BAD_ARG;
+    if (b == 0) return INVPREF_OK;
+    return launch_topk_stream(rows, row_ids, b, params->Uinv, desc->n_users, g.D, desc->implicit, nullptr, excl_off,
+                              excl_users, nullptr, nullptr, 1, nullptr, nullptr, k, top_users, top_scores, nullptr,
+                              nullptr, (cudaStream_t)stream);
+}
+
 int invpref_fetch_rows_p2p(const float* const* tables, int32_t world, const int32_t* owner, const int64_t* rows,
                            int64_t n, int32_t dim, float* out_inv, float* out_env, void* stream) {
     if (n < 0 || dim < 1 || !tables || (n > 0 && (!owner || !rows || !out_inv || !out_env))) return INVPREF_ERR_BAD_ARG;

@@ -180,6 +180,14 @@ int launch_topk_stream(const float* Q, const int64_t* qids, int64_t b, const flo
 // inv_norm[i] = 1 / sqrtf(sum_d x[i, d]^2) for the n rows of x [n, D] (row_inv_norm_kernel: order and edge cases)
 int launch_row_inv_norm(const float* x, int64_t n, int D, float* inv_norm, cudaStream_t stream);
 
+// ---- foldin.cu -------------------------------------------------------------------------------
+// fold-in of the b histories (off [b + 1], ids, scores) against the catalogue table V [n_cat, D]: fp32 rows out [b, D]
+// and Newton step counts iters [b] (nullable); the definition is invpref_fold_in_users' in the header
+int fold_in_max_dim();
+int launch_fold_in(const float* V, int64_t n_cat, int D, int implicit, const int64_t* off, const int64_t* ids,
+                   const float* scores, int64_t b, double l2, int max_iter, float* out, int32_t* iters,
+                   cudaStream_t stream);
+
 // ---- plan.cu ---------------------------------------------------------------------------------
 int build_plan_side(const int64_t* ids, const int64_t* other_ids, int64_t other_rows, const int32_t* other_seg_of,
                     PlanSide p, char* tmp, size_t tmp_bytes, cudaStream_t stream);

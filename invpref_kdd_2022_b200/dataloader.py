@@ -117,6 +117,23 @@ def user_item_csr(users: np.ndarray, items: np.ndarray, n_users: int):
     return np.cumsum(off), key % width
 
 
+def interaction_csr(rows: np.ndarray, cols: np.ndarray, scores: np.ndarray, n_rows: int):
+    """Interaction triples grouped by row as (offsets int64 [n_rows + 1], cols int64 [n], scores fp32 [n]): the
+    history format of ``fold_in_users`` (rows = new users, cols = items) and ``fold_in_items`` (rows = new items,
+    cols = users).  Stable: a row's entries keep their input order; duplicates are kept (each is an observation)."""
+    rows = np.asarray(rows, dtype=np.int64).reshape(-1)
+    cols = np.asarray(cols, dtype=np.int64).reshape(-1)
+    scores = np.asarray(scores, dtype=np.float32).reshape(-1)
+    if not (rows.size == cols.size == scores.size):
+        raise ValueError(f"rows, cols and scores differ in length: {rows.size}, {cols.size}, {scores.size}")
+    if rows.size and (rows.min() < 0 or rows.max() >= n_rows):
+        raise IndexError(f"row id outside [0, {n_rows})")
+    order = np.argsort(rows, kind="stable")
+    off = np.zeros(n_rows + 1, dtype=np.int64)
+    np.cumsum(np.bincount(rows, minlength=n_rows), out=off[1:])
+    return off, cols[order], scores[order]
+
+
 _csr = user_item_csr        # tests/test_gpu_drivers.py imports the earlier private name
 
 

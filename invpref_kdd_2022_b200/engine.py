@@ -414,6 +414,85 @@ class HotPath:
                                               _lib.ptr(top), _lib.ptr(sc), _lib.stream_ptr()), "top_users")
         return top, sc
 
+    def fold_in_users(self, off, items, scores, l2: float, max_iter: int = 25, return_iters: bool = False):
+        """``invpref_fold_in_users``: invariant rows (fp32 [b, D]) for users outside the table, from their histories
+        (``off`` int64 [b + 1], ``items`` int64, ``scores`` fp32: CUDA tensors, CSR), against the item table.  See
+        the header for the objective, the stopping rule and the edge cases.  ``l2`` > 0 is a per-row ridge
+        coefficient (no default: the training L2 term is a per-batch mean and does not map onto it).  Reads only the
+        item table: no flush.  ``return_iters``: also return the Newton step counts (int32 [b])."""
+        return self._fold_in("invpref_fold_in_users", self.n_items, off, items, scores, l2, max_iter, return_iters)
+
+    def fold_in_items(self, off, users, scores, l2: float, max_iter: int = 25, return_iters: bool = False):
+        """``invpref_fold_in_items``: ``fold_in_users`` for items outside the table, from (user, score) histories,
+        against the user table (flushed first in lazy mode)."""
+        self.flush()
+        return self._fold_in("invpref_fold_in_items", self.n_users, off, users, scores, l2, max_iter, return_iters)
+
+    def _fold_in(self, fn, n_cat, off, ids, scores, l2, max_iter, return_iters):
+        import math
+        if self.dim > _lib.FOLD_IN_MAX_DIM:
+            raise RuntimeError(f"fold-in supports D <= {_lib.FOLD_IN_MAX_DIM} (this model: D = {self.dim})")
+        l2, max_iter = float(l2), int(max_iter)
+        if not (math.isfinite(l2) and l2 > 0.0):
+            raise ValueError(f"l2 must be finite and > 0, got {l2}")
+        if max_iter < 1:
+            raise ValueError(f"max_iter must be >= 1, got {max_iter}")
+        off, ids, scores = (self._query_ids(t, fn[8:]) for t in (off, ids, scores))
+        if off.dtype != torch.int64 or ids.dtype != torch.int64 or scores.dtype != torch.float32 or off.dim() != 1 \
+                or ids.dim() != 1 or scores.dim() != 1 or off.numel() < 1 or ids.numel() != scores.numel():
+            raise ValueError(f"history: CSR (off int64 [b + 1], ids int64 [n], scores fp32 [n]) expected, got off "
+                             f"{off.dtype} {tuple(off.shape)}, ids {ids.dtype} {tuple(ids.shape)}, scores "
+                             f"{scores.dtype} {tuple(scores.shape)}")
+        b, n = off.numel() - 1, ids.numel()
+        # one host synchronisation: bit 0 = malformed offsets, bit 1 = an id outside the catalogue
+        flag = (off[0] != 0).to(torch.int32) | (off[-1] != n).to(torch.int32)
+        if b:
+            flag |= (off[1:] < off[:-1]).any().to(torch.int32)
+        if n:
+            flag |= ((ids < 0) | (ids >= n_cat)).any().to(torch.int32) * 2
+        f = int(flag.item())
+        if f & 1:
+            raise ValueError(f"history: offsets must start at 0, not decrease and end at len(ids) = {n}")
+        if f & 2:
+            raise IndexError(f"index out of range in self: history id outside its table ({n_cat} rows)")
+        rows = torch.empty((b, self.dim), dtype=torch.float32, device=self.device)
+        iters = torch.empty(b, dtype=torch.int32, device=self.device) if return_iters else None
+        if not n:                                             # empty histories: valid pointers
+            ids = torch.zeros(1, dtype=torch.int64, device=self.device)
+            scores = torch.zeros(1, dtype=torch.float32, device=self.device)
+        p = _lib.make_params(self.params)
+        _lib.check(getattr(self.lib, fn)(C.byref(self.desc), C.byref(p), _lib.ptr(off, torch.int64),
+                                         _lib.ptr(ids, torch.int64), _lib.ptr(scores, torch.float32), b, l2, max_iter,
+                                         _lib.ptr(rows), _lib.ptr(iters, torch.int32), _lib.stream_ptr()), fn[8:])
+        return (rows, iters) if return_iters else rows
+
+    def recommend_rows(self, rows, k: int, exclude=None):
+        """``invpref_recommend_rows``: ``recommend`` for the query rows ``rows`` (fp32 CUDA [b, D], e.g. from
+        ``fold_in_users``) -> (items int64 [b, k], scores fp32 [b, k]), bit for bit ``recommend``'s scores for a user
+        with that row.  ``exclude``: ``(off, items)`` CSR over the b rows.  Reads only the item table: no flush."""
+        return self._topk_rows("invpref_recommend_rows", rows, k, exclude)
+
+    def top_users_rows(self, rows, k: int, exclude=None):
+        """``invpref_top_users_rows``: ``top_users`` for the item rows ``rows`` (fp32 CUDA [b, D], e.g. from
+        ``fold_in_items``) -> (users int64 [b, k], scores fp32 [b, k]).  ``exclude``: ``(off, users)`` CSR over the b
+        rows.  Flushes lazy user rows first."""
+        self.flush()
+        return self._topk_rows("invpref_top_users_rows", rows, k, exclude)
+
+    def _topk_rows(self, fn, rows, k, exclude):
+        rows = self._query_ids(rows, fn[8:])
+        if rows.dtype != torch.float32 or rows.dim() != 2 or rows.shape[1] != self.dim:
+            raise ValueError(f"rows: fp32 [b, {self.dim}] expected, got {rows.dtype} {tuple(rows.shape)}")
+        b = rows.shape[0]
+        row_ids = torch.arange(b, dtype=torch.int64, device=self.device)
+        top, sc = self._topk_out(b, k)
+        e_off, e_ids = self._exclusion_csr(exclude, b, "rows")
+        p = _lib.make_params(self.params)
+        _lib.check(getattr(self.lib, fn)(C.byref(self.desc), C.byref(p), _lib.ptr(rows), _lib.ptr(row_ids), b,
+                                         _lib.ptr(e_off, torch.int64), _lib.ptr(e_ids, torch.int64), int(k),
+                                         _lib.ptr(top), _lib.ptr(sc), _lib.stream_ptr()), fn[8:])
+        return top, sc
+
     @staticmethod
     def _query_ids(ids, what):
         ids = ids.contiguous()

@@ -238,6 +238,41 @@ class _InvPref(nn.Module):
         hp = self.hot_path()
         return hp.top_users(_ids_on(items_id, hp.device), k, _csr_on(exclude, hp.device))
 
+    def fold_in_users(self, off, items, scores, l2: float, max_iter: int = 25, return_iters: bool = False):
+        """Invariant rows for users who are not in the table (signed up after training) -> fp32 [b, D], with the item
+        table fixed: row r minimises the model's own invariant loss over the user's history (items[off[r]:off[r+1]],
+        scores[...]) plus ``l2 / 2 * |u|^2`` -- ridge regression on the explicit model, logistic regression (damped
+        Newton, at most ``max_iter`` steps) on the implicit one -- in fp64 on the GPU, rounded to fp32 once.  Rank the
+        catalogue for the new users with ``recommend_rows``.  ``l2`` > 0 has no default: the training L2 term is a
+        per-batch mean and does not map onto a per-row ridge.  ``off`` / ``items`` / ``scores``: numpy arrays or
+        tensors, e.g. ``dataloader.interaction_csr(rows, items, scores, b)``.  An empty history gives the zero row; a
+        NaN / inf score or table row makes that row NaN.  ``return_iters``: also return the Newton step counts (int32
+        [b]; 1 on the explicit model, 0 for an empty history, ``-max_iter`` if the stopping rule was not met).  Ids
+        outside the item table raise IndexError."""
+        hp = self.hot_path()
+        return hp.fold_in_users(*_history_on(off, items, scores, hp.device), l2, max_iter, return_iters)
+
+    def fold_in_items(self, off, users, scores, l2: float, max_iter: int = 25, return_iters: bool = False):
+        """``fold_in_users`` for items that are not in the table (e.g. news published after training), from their
+        (user, score) histories, against the user table -> fp32 item rows [b, D] for ``top_users_rows``."""
+        hp = self.hot_path()
+        return hp.fold_in_items(*_history_on(off, users, scores, hp.device), l2, max_iter, return_iters)
+
+    def recommend_rows(self, rows, k: int, exclude=None):
+        """``recommend`` for user rows that are not in the table (e.g. from ``fold_in_users``): ``rows`` fp32 [b, D]
+        -> (items int64 [b, k], scores fp32 [b, k]); the scores are ``recommend``'s for a user with that row, bit for
+        bit.  ``exclude``: ``(off, items)`` CSR over the b rows (e.g. the history that was folded in)."""
+        hp = self.hot_path()
+        return hp.recommend_rows(torch.as_tensor(rows, dtype=torch.float32).to(hp.device), k,
+                                 _csr_on(exclude, hp.device))
+
+    def top_users_rows(self, rows, k: int, exclude=None):
+        """``top_users`` for item rows that are not in the table (e.g. from ``fold_in_items``): ``rows`` fp32 [b, D]
+        -> (users int64 [b, k], scores fp32 [b, k]).  ``exclude``: ``(off, users)`` CSR over the b rows."""
+        hp = self.hot_path()
+        return hp.top_users_rows(torch.as_tensor(rows, dtype=torch.float32).to(hp.device), k,
+                                 _csr_on(exclude, hp.device))
+
     def cluster_predict(self, users_id, items_id, envs_id) -> torch.Tensor:
         """models.py:541-543 / 409-411: env-aware score only (the classifier pass is skipped)."""
         hp = self.hot_path()
@@ -254,6 +289,13 @@ def _csr_on(csr, dev):
     if csr is None:
         return None
     return tuple(torch.as_tensor(np.ascontiguousarray(x) if isinstance(x, np.ndarray) else x).to(dev) for x in csr)
+
+
+def _history_on(off, ids, scores, dev):
+    """A fold-in history (off, ids, scores) of numpy arrays or tensors -> int64 / int64 / fp32 tensors on `dev`."""
+    off, ids = _csr_on((off, ids), dev)
+    scores = torch.as_tensor(np.ascontiguousarray(scores) if isinstance(scores, np.ndarray) else scores)
+    return off.to(torch.int64), ids.to(torch.int64), scores.to(dev, torch.float32)
 
 
 class BasicRecommender(nn.Module):
