@@ -785,7 +785,7 @@ int invpref_cluster_sorted(const invpref_desc* desc, const invpref_params* param
     a.old_envs = old_envs; a.B = N; a.D = g.D; a.K = g.K; a.implicit = desc->implicit;
     a.new_envs = new_envs; a.hist = (unsigned long long*)hist; a.diff = (unsigned long long*)diff;
     a.perm = perm; a.users32 = users_sorted; a.items32 = items_sorted;
-    return launch_cluster_sorted(g, a, (cudaStream_t)stream);
+    return launch_cluster(g, a, (cudaStream_t)stream);
 }
 
 int invpref_stat_envs(const int64_t* envs, int64_t N, int32_t n_envs, const int64_t* hist, float* class_weights,

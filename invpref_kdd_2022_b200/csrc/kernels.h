@@ -127,13 +127,12 @@ struct ClusterArgs {
     int D, K, implicit;
     int64_t* new_envs;
     unsigned long long *hist, *diff;
-    // user-sorted view (launch_cluster_sorted): sample k of the view is original sample perm[k]; users32 / items32 /
+    // user-sorted view (perm != nullptr): sample k of the view is original sample perm[k]; users32 / items32 /
     // scores are the sorted copies, perm_idx / old_envs / new_envs stay in original order
     const int32_t *perm, *users32, *items32;
 };
 
 int launch_cluster(const Geometry& g, const ClusterArgs& a, cudaStream_t stream);
-int launch_cluster_sorted(const Geometry& g, const ClusterArgs& a, cudaStream_t stream);
 int launch_env_hist(const int64_t* envs, int64_t N, int K, unsigned long long* hist, cudaStream_t stream);
 int launch_stat_envs(const int64_t* envs, int64_t N, int K, const int64_t* hist, float* class_weights,
                      float* sample_weights, cudaStream_t stream);

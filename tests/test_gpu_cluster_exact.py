@@ -69,7 +69,7 @@ def geometry(D, K):
 
 
 def stages(D, K):
-    """cluster.cu ClStages: ring depth."""
+    """cluster.cu cl_stages: ring depth."""
     vec, nv, _ = geometry(D, K)
     return 3 if vec * nv <= 8 else 2
 
